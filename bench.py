@@ -1,9 +1,18 @@
 """bench.py -- MPC solves/sec (H=20, 8 obstacles) on B200.  See DESIGN.md "Measurement".
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--n-starts S] [--config 1|2|3]
+                  [--dump-outputs DIR]
 
 --config 3 (default) is the headline workload; the same JSON line carries the other BASELINE configurations as extra
 keys (`single_start`, `config1_latency`, `config2`, and `config5` under --gpus N); --config 1 / 2 print only that one.
+--steps K sets the number of timed steps of every measurement except config 1 (--config 1 and the `config1_latency`
+key), whose timed region is the workload itself: the 100-call closed loop of the reference's run script.
+
+--dump-outputs DIR saves what the last timed step of the config-3 path computed (actions, cost, status, is_collide); the
+inputs depend only on the arguments, so two builds run with the same arguments can be compared output for output.
+Under --gpus N rank 0 writes its own shard: cost, status and is_collide exist only on the rank that solved those
+problems, and rank 0's part of the gathered actions is its local actions.  Configs 1 and 2 and --impl reference are
+not dumped (--dump-outputs is refused there).
 
 One "step" = one full predict (parse -> collision check -> regeneration -> solve to convergence ->
 first control) over one batch of synthetic intersection scenarios (BASELINE config 3: 65536
@@ -228,6 +237,29 @@ def timed_steps(torch, fn, steps, warmup=3):
     return e0.elapsed_time(e1) / steps
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+NPY_HEADER_BYTES = 128          # the .npy header numpy writes for a short dtype / shape description
+
+
+def dump_outputs(out_dir: str, tensors) -> None:
+    """Saves per-problem outputs as float32 (status codes and flags are small integers, exact in float32).  When the
+    files, headers included, would exceed DUMP_LIMIT_BYTES, a fixed seeded sample of problems is kept and its indices
+    go to sample_index.npy (float64)."""
+    import numpy as np
+    arrays = {k: v.cpu().numpy().astype(np.float32) for k, v in tensors.items()}
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes + len(arrays) * NPY_HEADER_BYTES > DUMP_LIMIT_BYTES:
+        row_bytes += 8                                                   # + sample_index
+        n_keep = (DUMP_LIMIT_BYTES - (len(arrays) + 1) * NPY_HEADER_BYTES) // row_bytes
+        idx = np.sort(np.random.default_rng(0).choice(n, n_keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["sample_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -241,12 +273,17 @@ def main() -> None:
     ap.add_argument("--n-starts", type=int, default=0, help="start portfolio size (0 = library default, 4; 1 = the reference's cold start only)")
     ap.add_argument("--config", type=int, default=3, choices=(1, 2, 3), help="BASELINE configuration to print (3 = headline)")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra keys (single_start, config1_latency, config2, config5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (actions, cost, status, is_collide; rank 0's shard) "
+                         "as DIR/<name>.npy, for comparing the outputs of two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config != 3):
+        ap.error("--dump-outputs applies to the config-3 path of --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
-        if args.steps > 8:
-            args.steps = 8
         run_reference(args)
         return
 
@@ -336,6 +373,10 @@ def main() -> None:
     kt = agent.timing_end()
     launches = agent.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # taken before the e2e pass below reuses the agent's output buffers
+        dump_outputs(args.dump_outputs, {"actions": agent.actions[:B], "cost": agent.cost[:B], "status": agent.status[:B],
+                                         "is_collide": agent.is_collide[:B]})
     it = agent.iters[:B].float()
     st = agent.status[:B]
     mean_iters = float(it.mean())
@@ -456,7 +497,7 @@ def main() -> None:
                 o, r = dev_batches[i % n_unique]
                 a1.reset()
                 a1.predict_batch(o, ref_speed=r)
-            ms1 = timed_steps(torch, s1, min(args.steps, 10))
+            ms1 = timed_steps(torch, s1, args.steps)
             st1 = a1.status[:B]
             extras["single_start"] = {"n_starts": 1, "value": B / (ms1 * 1e-3), "unit": "solves/s", "ms_per_step": ms1,
                                       "mean_iters": float(a1.iters[:B].float().mean()),
@@ -466,7 +507,7 @@ def main() -> None:
             a1.close()
         if world == 1:
             extras["config1_latency"] = config1_latency(pkg, local, args.n_starts)
-            extras["config2"] = config2(pkg, torch, local, args.n_starts, min(args.steps, 10))
+            extras["config2"] = config2(pkg, torch, local, args.n_starts, args.steps)
 
     line = {"metric": "mpc_solves_per_sec", "value": value, "unit": "solves/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak",

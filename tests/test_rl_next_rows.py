@@ -99,7 +99,6 @@ def test_gsde_likelihood_matches_sampling_cpu():
 
 
 def test_sb3_zip_checkpoints_cpu(tmp_path):
-    import os
     from mpc_rl_for_avs_b200 import checkpoint
     from mpc_rl_for_avs_b200.rl import ActorCritic
     torch.manual_seed(1)
@@ -111,14 +110,71 @@ def test_sb3_zip_checkpoints_cpu(tmp_path):
         assert pol2.use_sde == use_sde and data["n_steps"] == 64
         x = torch.randn(5, 80)
         assert torch.equal(pol(x, deterministic=True)[0], pol2(x, deterministic=True)[0])
-    # the reference's own checkpoints (A2C: state-independent std; PPO: gSDE), when the reference tree is present
-    ref = "/root/reference/weights/v0"
-    if os.path.isdir(ref):
-        for name, sde in (("test_a2c_v0.zip", False), ("test_ppo_v0.zip", True)):
-            pol, data = checkpoint.load_sb3_policy(os.path.join(ref, name))
-            assert pol.use_sde == sde and data["observation_space_shape"] == (10, 8) and data["action_space_shape"] == (1,)
-            a, v, lp = pol(torch.zeros(3, 80), deterministic=True)
-            assert a.shape == (3, 1) and torch.isfinite(a).all() and torch.isfinite(v).all()
+    # checkpoints as Stable-Baselines3 writes the reference's (weights/v0: A2C with a state-independent std, PPO with
+    # gSDE): the parameter names and shapes of SB3's MlpPolicy are spelled out below, not taken from ActorCritic, and the
+    # loaded policy must compute what that MlpPolicy computes
+    rng = np.random.default_rng(5)
+    x = rng.standard_normal((5, 10, 8))
+    for name, sde, hp in (("test_a2c_v0.zip", False, {"n_steps": 64, "learning_rate": 0.0007, "num_timesteps": 128}),
+                          ("test_ppo_v0.zip", True, {"n_steps": 64, "batch_size": 64, "n_epochs": 10, "num_timesteps": 256})):
+        sd = _sb3_mlp_policy_state(rng, 80, 1, sde)
+        path = str(tmp_path / name)
+        _write_sb3_layout_zip(path, sd, sde, hp)
+        pol, data = checkpoint.load_sb3_policy(path)
+        assert pol.use_sde == sde and data["observation_space_shape"] == (10, 8) and data["action_space_shape"] == (1,)
+        assert all(data[k] == v for k, v in hp.items()) and "policy_class" not in data and "lr_schedule" not in data
+        a, v, lp = pol(torch.zeros(3, 80), deterministic=True)
+        assert a.shape == (3, 1) and torch.isfinite(a).all() and torch.isfinite(v).all()
+        a, v, _ = pol(torch.from_numpy(x.reshape(5, 80)).float(), deterministic=True)
+        a_ref, v_ref = _sb3_mlp_forward(sd, x.reshape(5, 80))
+        assert np.allclose(a.detach().numpy(), a_ref, rtol=0, atol=1e-5) and np.allclose(v.detach().numpy(), v_ref, rtol=0, atol=1e-5)
+
+
+def _sb3_mlp_policy_state(rng, obs_dim, action_dim, use_sde):
+    """policy.pth of SB3's ActorCriticPolicy as A2C / PPO save it with the reference's defaults, filled with seeded
+    values: FlattenExtractor (no parameters), net_arch pi=[64, 64] / vf=[64, 64] as Sequential(Linear, Tanh, Linear, Tanh),
+    the action_net / value_net heads, log_std [action_dim] (diagonal Gaussian) or [64, action_dim] (gSDE, full_std)."""
+    shapes = {"log_std": (64, action_dim) if use_sde else (action_dim,)}
+    for tower in ("policy_net", "value_net"):
+        shapes.update({f"mlp_extractor.{tower}.0.weight": (64, obs_dim), f"mlp_extractor.{tower}.0.bias": (64,),
+                       f"mlp_extractor.{tower}.2.weight": (64, 64), f"mlp_extractor.{tower}.2.bias": (64,)})
+    shapes.update({"action_net.weight": (action_dim, 64), "action_net.bias": (action_dim,),
+                   "value_net.weight": (1, 64), "value_net.bias": (1,)})
+    return {k: torch.from_numpy(rng.uniform(-0.3, 0.3, s).astype(np.float32)) for k, s in shapes.items()}
+
+
+def _sb3_mlp_forward(sd, x):
+    """Deterministic action (the Gaussian mean) and value of SB3's MlpPolicy for flattened observations, float64."""
+    p = {k: v.double().numpy() for k, v in sd.items()}
+
+    def tower(name):
+        h = np.tanh(x @ p[f"mlp_extractor.{name}.0.weight"].T + p[f"mlp_extractor.{name}.0.bias"])
+        return np.tanh(h @ p[f"mlp_extractor.{name}.2.weight"].T + p[f"mlp_extractor.{name}.2.bias"])
+    return tower("policy_net") @ p["action_net.weight"].T + p["action_net.bias"], \
+        (tower("value_net") @ p["value_net.weight"].T + p["value_net.bias"])[:, 0]
+
+
+def _write_sb3_layout_zip(path, state_dict, use_sde, hyper):
+    """A checkpoint in the member layout and `data` format of Stable-Baselines3's `model.save` (gymnasium Box spaces;
+    the cloudpickled class and schedule entries stand in as opaque strings)."""
+    import io
+    import json
+    import zipfile
+
+    def box(shape, low, high):
+        return {":type:": "<class 'gymnasium.spaces.box.Box'>", ":serialized:": "gAWV-opaque-", "dtype": "float32",
+                "_shape": list(shape), "low_repr": low, "high_repr": high, "_np_random": None}
+    data = {"policy_class": {":type:": "<class 'abc.ABCMeta'>", ":serialized:": "gAWV-opaque-",
+                             "__module__": "stable_baselines3.common.policies"},
+            "observation_space": box((10, 8), "-inf", "inf"), "action_space": box((1,), "-1.0", "1.0"),
+            "lr_schedule": {":type:": "<class 'function'>", ":serialized:": "gAWV-opaque-"},
+            "use_sde": use_sde, "sde_sample_freq": -1, "gamma": 0.99, "n_envs": 1, **hyper}
+    buf = io.BytesIO()
+    torch.save(state_dict, buf)
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_DEFLATED) as z:
+        z.writestr("data", json.dumps(data, indent=4))
+        z.writestr("policy.pth", buf.getvalue())
+        z.writestr("_stable_baselines3_version", "2.3.2")
 
 
 def test_evaluation_harness_cpu():
