@@ -174,6 +174,18 @@ MPC_API int mpc_predict(MpcHandle* h, const float* obs, const float* ref_speed, 
  * A warm start changes which local optimum of the multi-modal NLP is found: keep it off for parity runs. */
 MPC_API int mpc_set_warm_start(MpcHandle* h, const float* u_init);
 
+/* OPT-IN adaptive portfolio: subsequent mpc_solve / mpc_predict(_host) calls run starts n_starts..max_starts-1 only for
+ * problems whose base objectives J_0..J_{n_starts-1} disagree: any of them not finite, or
+ * max J - min J > rel_gap * max(|min J|, 1).  Such a problem is "extended"; its results (actions, status, cost, U, iters)
+ * are bit-identical to those of a handle with n_starts = max_starts, every other problem's to those of this handle without
+ * the mode.  The extra starts are queued inside the running solve launch by the thread that finishes a problem's last
+ * base start, so the mode costs no second launch; it may lengthen the launch's tail by up to one more solve.
+ * Needs the handle's n_starts >= 2 and max_starts in (n_starts, MPC_MAX_STARTS]; rel_gap must not be NaN (+inf: extend
+ * only problems with a non-finite base objective; < 0: extend all).  max_starts = 0 switches the mode off.
+ * start_cost [max_starts][max_batch] (row stride max_batch; NaN for starts that did not run) and extended [B] are device
+ * pointers or NULL, borrowed until replaced.  Allocates; do not call during stream capture. */
+MPC_API int mpc_set_adaptive_starts(MpcHandle* h, int max_starts, float rel_gap, float* start_cost, uint8_t* extended);
+
 /* Same call with HOST buffers (what a numpy caller holds): obs/ref_speed/weights/reset_mask are
  * copied host->device, actions/status (and is_collide) device->host, inside the call; the latch
  * lives in the handle.  col_host (may be NULL, and so may any pointer in it) receives the per-call collision
@@ -194,7 +206,8 @@ MPC_API int mpc_fp32_peak(MpcHandle* h, int repeats, float* tflops_out);
 MPC_API int mpc_timing_begin(MpcHandle* h);
 MPC_API int mpc_timing_end(MpcHandle* h, float* prepare_ms_avg, float* solve_ms_avg, int* n_prepare, int* n_solve);
 /* which solve kernel a launch of B problems uses: *gains_in_tmem = 1 -> k_solve_tmem (feedback gains in
- * tensor memory), 0 -> k_solve (gains in shared memory); *threads_per_block = its block size (one block per SM) */
+ * tensor memory), 0 -> k_solve (gains in shared memory); *threads_per_block = its block size (one block per SM).
+ * The launch is sized on the B * n_starts base work items; the adaptive portfolio's extra starts do not change it. */
 MPC_API int mpc_solve_config(const MpcHandle* h, int B, int* gains_in_tmem, int* threads_per_block);
 /* device properties used for grid sizing */
 MPC_API int mpc_device_info(const MpcHandle* h, int* sm_count, int* cc_major, int* cc_minor, int* smem_per_block_optin);

@@ -69,7 +69,8 @@ class MpcEnvStep(C.Structure):
 
 EXPORTS = ["mpc_create", "mpc_destroy", "mpc_last_error", "mpc_workspace_batch", "mpc_rollout_cost", "mpc_solve",
            "mpc_prepare", "mpc_predict", "mpc_predict_host", "mpc_launch_count", "mpc_fp32_peak", "mpc_timing_begin",
-           "mpc_timing_end", "mpc_device_info", "mpc_set_warm_start", "mpc_solve_config", "mpc_env_step"]
+           "mpc_timing_end", "mpc_device_info", "mpc_set_warm_start", "mpc_set_adaptive_starts", "mpc_solve_config",
+           "mpc_env_step"]
 
 
 class MpcError(RuntimeError):
@@ -113,6 +114,8 @@ def load() -> C.CDLL:
     lib.mpc_predict_host.restype = C.c_int
     lib.mpc_set_warm_start.argtypes = [vp, vp]
     lib.mpc_set_warm_start.restype = C.c_int
+    lib.mpc_set_adaptive_starts.argtypes = [vp, C.c_int, C.c_float, vp, vp]
+    lib.mpc_set_adaptive_starts.restype = C.c_int
     lib.mpc_launch_count.argtypes = [vp]
     lib.mpc_launch_count.restype = C.c_int64
     lib.mpc_fp32_peak.argtypes = [vp, C.c_int, C.POINTER(C.c_float)]

@@ -54,7 +54,13 @@ class BatchedPureMPC:
     n_starts: the NLP is multi-modal, so every problem is solved from `n_starts` starts (0 = the library default, 4)
     and the lowest objective wins; start 0 is the reference's own cold start (zero controls,
     agents/pure_mpc.py:244) and `n_starts=1` solves only that one (about 2.5x the throughput); `n_starts=2` adds the
-    path-following start that finds the best optimum most often (DESIGN.md 2)."""
+    path-following start that finds the best optimum most often (DESIGN.md 2).
+
+    `set_adaptive_starts(max_starts, rel_gap)` (opt-in) runs starts n_starts..max_starts-1 only for the problems whose
+    first n_starts objectives disagree: most of the J_gpu <= J_oracle gain of max_starts starts for a fraction of their
+    solves.  It trades a longer launch tail (a problem whose last base start ends late adds its extra solves at the end)
+    for the solves skipped on problems where the base starts agree; each problem's result is bit-identical to a fixed
+    portfolio of n_starts or max_starts starts."""
 
     def __init__(self, cfg: Dict, vehicles_count: int, max_batch: int, device: Union[int, str, torch.device] = 0,
                  dt: float = 0.1, collision_check: bool = True, literal_no_collision: bool = False,
@@ -109,6 +115,9 @@ class BatchedPureMPC:
         self.conflict_point = torch.full((B, M, 2), float("nan"), dtype=torch.float32, device=dev)
         self.reference_trajectory = torch.from_numpy(reference_path(self.dt)[:, :2].copy()).to(dev)
         self._u_init = None
+        self.max_starts = 0
+        self.start_cost = None
+        self.extended = None
 
     # ------------------------------------------------------------------ lifecycle
     def close(self) -> None:
@@ -197,6 +206,31 @@ class BatchedPureMPC:
             raise ValueError(f"u_init must be [B, {self.horizon}, 2]")
         self._u_init = u
         _capi.check(self._lib, self._h, self._lib.mpc_set_warm_start(self._h, u.data_ptr()))
+
+    def set_adaptive_starts(self, max_starts: Optional[int], rel_gap: float = 1e-3) -> None:
+        """OPT-IN adaptive portfolio: the next solves run starts n_starts..max_starts-1 only for problems whose first
+        n_starts objectives disagree (one not finite, or max - min > rel_gap * max(|min|, 1)); the others keep the
+        n_starts result.  After a call of B problems, `self.start_cost[:, :B]` holds every start's objective (NaN where
+        a start did not run) and `self.extended[:B]` marks the problems that ran the extra starts.  None or 0 switches
+        the mode off.  Allocates: call it outside CUDA graph capture."""
+        if max_starts is None or int(max_starts) == 0:
+            _capi.check(self._lib, self._h, self._lib.mpc_set_adaptive_starts(self._h, 0, 0.0, None, None))
+            self.max_starts, self.start_cost, self.extended = 0, None, None
+            return
+        S = int(max_starts)
+        if self.n_starts < 2:
+            raise ValueError("the adaptive portfolio needs n_starts >= 2")
+        if not self.n_starts < S <= _capi.MAX_STARTS:
+            raise ValueError(f"max_starts must be in ({self.n_starts}, {_capi.MAX_STARTS}], got {S}")
+        if math.isnan(float(rel_gap)):
+            raise ValueError("rel_gap must not be NaN")
+        if self.max_batch * S > 0x7FFFFFFF // 64:
+            raise ValueError("max_batch * max_starts too large")
+        start_cost = torch.full((S, self.max_batch), float("nan"), dtype=torch.float32, device=self.device)
+        extended = torch.zeros(self.max_batch, dtype=torch.uint8, device=self.device)
+        rc = self._lib.mpc_set_adaptive_starts(self._h, S, float(rel_gap), start_cost.data_ptr(), extended.data_ptr())
+        _capi.check(self._lib, self._h, rc)
+        self.max_starts, self.start_cost, self.extended = S, start_cost, extended
 
     @staticmethod
     def shift_controls(U: torch.Tensor) -> torch.Tensor:

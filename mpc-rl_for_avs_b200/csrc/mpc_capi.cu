@@ -33,6 +33,14 @@ struct MpcHandle {
   int* work_counter = nullptr;
   int n_starts = 1;
   SolveCand cand{};                // candidate results of the start portfolio (n_starts > 1)
+  int cand_starts = 0;             // starts the candidate arrays hold per problem (n_starts, or max_starts once adaptive)
+  // opt-in adaptive portfolio (mpc_set_adaptive_starts); max_starts = 0: off
+  int max_starts = 0;
+  float rel_gap = 0.f;
+  int* aq_block = nullptr;         // [2 + max_batch + (aq_starts - n_starts) * max_batch]: reserve, items_done, base_done, extra
+  int aq_starts = 0;
+  float* start_cost = nullptr;     // borrowed
+  uint8_t* extended = nullptr;     // borrowed
   const float* u_init = nullptr;   // opt-in warm start (device, borrowed)
   float* sink = nullptr;
   // host-call staging (mpc_predict_host)
@@ -76,7 +84,7 @@ MPC_API int mpc_destroy(MpcHandle* h) {
   cudaSetDevice(h->device);
   for (auto e : h->ev_prepare) cudaEventDestroy(e);
   for (auto e : h->ev_solve) cudaEventDestroy(e);
-  cudaFree(h->ws_block); cudaFree(h->work_counter); cudaFree(h->sink);
+  cudaFree(h->ws_block); cudaFree(h->work_counter); cudaFree(h->sink); cudaFree(h->aq_block);
   cudaFree(h->cand.cost); cudaFree(h->cand.u0); cudaFree(h->cand.status); cudaFree(h->cand.iters); cudaFree(h->cand.U);
   cudaFree(h->d_obs); cudaFree(h->d_ref_speed); cudaFree(h->d_weights); cudaFree(h->d_reset);
   cudaFree(h->d_actions); cudaFree(h->d_status); cudaFree(h->d_iters); cudaFree(h->d_cost);
@@ -205,6 +213,7 @@ MPC_API int mpc_create(const MpcConfig* cfg, int device, int max_batch, MpcHandl
     CKC(cudaMalloc(&h->cand.status, W * 4));
     CKC(cudaMalloc(&h->cand.iters, W * 4));
     CKC(cudaMalloc(&h->cand.U, W * (size_t)N * 8));
+    h->cand_starts = n_starts;
   }
   CKC(cudaMalloc(&h->sink, 256));
   // staging for the host-buffer entry point
@@ -344,11 +353,23 @@ MPC_API int mpc_solve(MpcHandle* h, const MpcProblemBatch* batch, int B, const M
   s.cfg = h->scfg; s.batch = *batch; s.out = *out; s.B = B; s.work_counter = h->work_counter;
   s.n_starts = h->n_starts; s.cand = h->cand;
   s.u_init = h->u_init;
+  s.aq = AdaptiveQueue{};
+  s.start_cost = nullptr; s.extended = nullptr; s.ld = h->max_batch;
+  if (h->max_starts > 0) {   // per-launch queue state: counters zeroed, extra list preset to -1 (all on the stream: capturable)
+    const size_t n_extra = (size_t)(h->max_starts - h->n_starts) * B;
+    s.aq.reserve = h->aq_block; s.aq.items_done = h->aq_block + 1; s.aq.base_done = h->aq_block + 2;
+    s.aq.extra = h->aq_block + 2 + h->max_batch;
+    s.aq.max_starts = h->max_starts; s.aq.rel_gap = h->rel_gap;
+    s.start_cost = h->start_cost; s.extended = h->extended;
+    CK(h, cudaMemsetAsync(h->aq_block, 0, (2 + (size_t)B) * sizeof(int), st));
+    CK(h, cudaMemsetAsync(s.aq.extra, 0xff, n_extra * sizeof(int), st));
+  }
   pick_solve_launch(h, B * h->n_starts, s);
   if ((rc = timed_begin(h, h->ev_solve, st))) return rc;
   CK(h, s.use_tmem ? launch_solve_tmem(s, st) : launch_solve(s, st));
   h->launches += 1;
-  if (h->n_starts > 1) { CK(h, launch_select(s, st)); h->launches += 1; }
+  if (h->max_starts > 0) { CK(h, launch_select_adaptive(s, st)); h->launches += 1; }
+  else if (h->n_starts > 1) { CK(h, launch_select(s, st)); h->launches += 1; }
   if ((rc = timed_end(h, h->ev_solve, st))) return rc;
   return MPC_OK;
 }
@@ -474,6 +495,47 @@ MPC_API int mpc_predict_host(MpcHandle* h, const float* obs_host, const float* r
 MPC_API int mpc_set_warm_start(MpcHandle* h, const float* u_init) {
   if (!h) return MPC_ERR_BAD_ARG;
   h->u_init = u_init;
+  return MPC_OK;
+}
+
+MPC_API int mpc_set_adaptive_starts(MpcHandle* h, int max_starts, float rel_gap, float* start_cost, uint8_t* extended) {
+  if (!h) return MPC_ERR_BAD_ARG;
+  if (max_starts == 0) {
+    h->max_starts = 0; h->start_cost = nullptr; h->extended = nullptr;
+    return MPC_OK;
+  }
+  if (h->n_starts < 2) return fail(h, MPC_ERR_BAD_ARG, "mpc_set_adaptive_starts: the handle's n_starts must be at least 2");
+  if (max_starts <= h->n_starts || max_starts > MPC_MAX_STARTS)
+    return fail(h, MPC_ERR_BAD_ARG, "mpc_set_adaptive_starts: max_starts must be in (n_starts, 8]");
+  if (rel_gap != rel_gap) return fail(h, MPC_ERR_BAD_ARG, "mpc_set_adaptive_starts: rel_gap is NaN");
+  if ((long long)h->max_batch * max_starts > 0x7fffffffLL / 64) return fail(h, MPC_ERR_BAD_ARG, "mpc_set_adaptive_starts: max_batch * max_starts too large");
+  CK(h, cudaSetDevice(h->device));
+  const size_t B = (size_t)h->max_batch;
+  if (max_starts > h->cand_starts) {     // candidate arrays for every start that may run; cudaFree waits for work in flight
+    SolveCand c{};
+    const size_t W = B * (size_t)max_starts;
+    cudaError_t e = cudaMalloc(&c.cost, W * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&c.u0, W * 8);
+    if (e == cudaSuccess) e = cudaMalloc(&c.status, W * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&c.iters, W * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&c.U, W * (size_t)h->scfg.N * 8);
+    SolveCand& old = e == cudaSuccess ? h->cand : c;
+    cudaFree(old.cost); cudaFree(old.u0); cudaFree(old.status); cudaFree(old.iters); cudaFree(old.U);
+    if (e != cudaSuccess) return fail(h, MPC_ERR_CUDA, "mpc_set_adaptive_starts: candidate arrays", e);
+    h->cand = c;
+    h->cand_starts = max_starts;
+  }
+  if (max_starts > h->aq_starts) {
+    int* q = nullptr;
+    CK(h, cudaMalloc(&q, (2 + B + (size_t)(max_starts - h->n_starts) * B) * sizeof(int)));
+    cudaFree(h->aq_block);
+    h->aq_block = q;
+    h->aq_starts = max_starts;
+  }
+  h->max_starts = max_starts;
+  h->rel_gap = rel_gap;
+  h->start_cost = start_cost;
+  h->extended = extended;
   return MPC_OK;
 }
 

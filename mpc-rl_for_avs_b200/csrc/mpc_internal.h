@@ -54,12 +54,24 @@ struct SolveCand {
   int32_t* iters;         // [S * B]
   float* U;               // [S * B][N][2]
 };
+// Adaptive portfolio (mpc_set_adaptive_starts): the base items (start < n_starts) are the tickets below B * n_starts;
+// the lane that finishes a problem's last base start appends that problem's extra items (starts n_starts..max_starts-1)
+// to `extra` when the base objectives disagree, and a larger ticket t takes slot t - B * n_starts of that list.
+// Zeroed / preset to -1 before every launch.
+struct AdaptiveQueue {
+  int* base_done;         // [B] base starts finished per problem; ends at n_starts, or n_starts + 1 when extended
+  int* extra;             // [(max_starts - n_starts) * B] extra items (start * B + problem), -1 = not written yet
+  int* reserve;           // slots of `extra` reserved so far
+  int* items_done;        // base items finished (each increments it after its publishing)
+  int max_starts;         // 0 = fixed portfolio
+  float rel_gap;
+};
 struct SolveLaunch {
   SolverConfig cfg;
   MpcProblemBatch batch;
   MpcSolveOut out;
   int B;                  // problems
-  int n_starts;           // work items = B * n_starts
+  int n_starts;           // work items = B * n_starts (base items of the adaptive portfolio)
   SolveCand cand;         // used when n_starts > 1
   int* work_counter;      // device, zeroed before launch
   const float* u_init;    // [B][N][2] warm start of start 0, or null
@@ -67,6 +79,10 @@ struct SolveLaunch {
   int grid;
   size_t smem_bytes;
   int use_tmem;           // gains in tensor memory (k_solve_tmem) instead of shared memory (k_solve)
+  AdaptiveQueue aq;       // aq.max_starts > 0: adaptive portfolio
+  float* start_cost;      // adaptive: [max_starts][ld] per-start objectives or null
+  uint8_t* extended;      // adaptive: [B] or null
+  int ld;                 // row stride of start_cost
 };
 cudaError_t launch_solve(const SolveLaunch& s, cudaStream_t stream);
 cudaError_t launch_rollout_cost(const SolverConfig& cfg, const MpcProblemBatch& batch, int B, const float* U,
@@ -78,5 +94,6 @@ size_t solve_smem_bytes_tmem(int N, int M, int tpb);
 bool tmem_layout_fits(int N, int tpb);
 cudaError_t launch_solve_tmem(const SolveLaunch& s, cudaStream_t stream);
 cudaError_t launch_select(const SolveLaunch& s, cudaStream_t stream);
+cudaError_t launch_select_adaptive(const SolveLaunch& s, cudaStream_t stream);
 
 }  // namespace mpcb

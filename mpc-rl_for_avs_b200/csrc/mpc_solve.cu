@@ -152,15 +152,63 @@ __device__ __forceinline__ void finish_item(const SolverConfig& cfg, const MpcSo
   }
 }
 
+// ---- adaptive portfolio: the work queue grows while the launch runs ---------------------------------------------
+// A ticket below B * S0 is base item `ticket`; a larger one reads slot ticket - B * S0 of the extra list.  Returns the
+// item, kTicketPending (slot not written yet and base items still running: poll again next trip -- never spin inside a
+// trip, the sweeps are warp-collective) or kTicketEmpty (definitively nothing left).
+constexpr int kTicketPending = -1, kTicketEmpty = -2;
+__device__ __forceinline__ int ld_acquire(const int* p) {
+  int v;
+  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ int poll_ticket(const AdaptiveQueue& aq, int B, int n_starts, int ticket) {
+  const int n_base = B * n_starts;
+  if (ticket < n_base) return ticket;
+  const int slot = ticket - n_base;
+  if (slot >= (aq.max_starts - n_starts) * B) return kTicketEmpty;   // past the list's capacity: can never be written
+  // every base item publishes before it counts itself finished: once all are counted, every reserved slot is written
+  const bool all_done = ld_acquire(aq.items_done) == n_base;
+  const int v = ld_acquire(aq.extra + slot);
+  if (v >= 0) return v;
+  if (all_done && slot >= ld_acquire(aq.reserve)) return kTicketEmpty;
+  return kTicketPending;
+}
+// After a base item's candidate is written: count it; the lane that finishes a problem's last base start reads the
+// S0 objectives and appends starts S0..S-1 when any is not finite or max - min > rel_gap * max(|min|, 1).
+__device__ __forceinline__ void publish_base(const AdaptiveQueue& aq, const SolveCand& cand, int B, int n_starts, int idx) {
+  const int b = idx % B;
+  __threadfence();                                           // the candidate before the count
+  if (atomicAdd(aq.base_done + b, 1) == n_starts - 1) {
+    __threadfence();
+    float lo = __ldcg(cand.cost + b), hi = lo;               // L2: the other starts were written by other SMs
+    bool finite = isfinite(lo);
+    for (int st = 1; st < n_starts; ++st) {
+      const float J = __ldcg(cand.cost + (size_t)st * B + b);
+      finite = finite && isfinite(J);
+      lo = fminf(lo, J); hi = fmaxf(hi, J);
+    }
+    if (!finite || hi - lo > aq.rel_gap * fmaxf(fabsf(lo), 1.f)) {
+      const int n_extra = aq.max_starts - n_starts;
+      const int r = atomicAdd(aq.reserve, n_extra);
+      for (int j = 0; j < n_extra; ++j) aq.extra[r + j] = (n_starts + j) * B + b;
+      aq.base_done[b] = n_starts + 1;                        // marks the problem extended for k_select_adaptive
+      __threadfence();
+    }
+  }
+  atomicAdd(aq.items_done, 1);
+}
+
 // One trip of the loop = [fetch] -> backward sweep -> line-search passes -> commit sweep -> bookkeeping,
 // each with exactly ONE call site so the kernel body stays near the instruction-cache size (the
 // first profile showed 2.3 stall cycles per issued instruction waiting for instructions).
 // A freshly fetched problem joins at the commit sweep (its first rollout is the commit under a zero
 // policy) and starts iterating on the next trip.
-template <int TPB>
+// kAdaptive: the adaptive portfolio (AdaptiveQueue); a lane whose ticket is not resolved yet is `pending`.
+template <int TPB, bool kAdaptive>
 __global__ void __launch_bounds__(TPB, 1)
 k_solve(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut out, const int B, int* __restrict__ work_counter,
-        const float* __restrict__ u_init, const int n_starts, const SolveCand cand) {
+        const float* __restrict__ u_init, const int n_starts, const SolveCand cand, const AdaptiveQueue aq) {
   extern __shared__ __align__(16) float smem[];
   const RefTab<float> ref = stage_tables(smem);
   using SL = Slots<float, true, TPB>;
@@ -170,19 +218,37 @@ k_solve(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut o
   ProblemScalars<float> p;
   SolveState<float> s;
   int idx = -1;
-  bool active = false, fresh = false, need_fetch = true;
+  bool active = false, fresh = false, need_fetch = true, pending = false;
 
   for (;;) {
     if (need_fetch) {
       need_fetch = false;
       idx = atomicAdd(work_counter, 1);
-      active = idx < B * n_starts;
-      if (active) {
-        begin_item(cfg, batch, B, idx, u_init, p, sl, s, ref);
-        fresh = true;
+      if constexpr (kAdaptive) {
+        pending = true;
+      } else {
+        active = idx < B * n_starts;
+        if (active) {
+          begin_item(cfg, batch, B, idx, u_init, p, sl, s, ref);
+          fresh = true;
+        }
       }
     }
-    if (!__any_sync(full, active)) break;
+    if constexpr (kAdaptive) {
+      if (pending) {
+        const int r = poll_ticket(aq, B, n_starts, idx);
+        if (r != kTicketPending) {
+          pending = false;
+          active = r >= 0;
+          if (active) {
+            idx = r;
+            begin_item(cfg, batch, B, idx, u_init, p, sl, s, ref);
+            fresh = true;
+          }
+        }
+      }
+    }
+    if (!__any_sync(full, active || pending)) break;
     float d1 = 0.f, d2 = 0.f, alpha = 1.f, Jn = 0.f, md = 0.f;
     bool acc = false;
     const bool run = active && !fresh;
@@ -205,6 +271,7 @@ k_solve(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut o
         after_line_search(cfg, s, acc, alpha, Jn, md, alpha * d1 + alpha * alpha * d2);
         if (s.done) {
           finish_item(cfg, out, cand, n_starts, idx, sl, s);
+          if constexpr (kAdaptive) if (idx < B * n_starts) publish_base(aq, cand, B, n_starts, idx);
           active = false;
           need_fetch = true;
         }
@@ -246,10 +313,10 @@ bool tmem_layout_fits(int N, int tpb) {
 #define MPC_SPEC_MAXK 8
 #endif
 
-template <int TPB>
+template <int TPB, bool kAdaptive>
 __global__ void __launch_bounds__(TPB, 1)
 k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut out, const int B, int* __restrict__ work_counter,
-             const float* __restrict__ u_init, const int n_starts, const SolveCand cand) {
+             const float* __restrict__ u_init, const int n_starts, const SolveCand cand, const AdaptiveQueue aq) {
   extern __shared__ __align__(16) float smem[];
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + kTabFloats);
   const int warp = threadIdx.x >> 5;
@@ -283,6 +350,7 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
   s.J = 0.f; s.mu = 0.f; s.hs = 1.f; s.J_mark = 0.f; s.md_last = 1e30f; s.iter = 0; s.status = 0; s.trials = 0; s.fails = 0; s.done = true;
   int idx = -1;
   bool active = false, fresh = false, need_fetch = true, first_wave = true;
+  bool pending = false;                                     // kAdaptive: holds a ticket whose slot is not written yet
 
   for (;;) {
     if (need_fetch) {
@@ -291,12 +359,32 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
       // atomics on one counter, and a small launch lands in the lowest lanes of every block; later: the shared queue
       idx = first_wave ? (int)(blockIdx.x + gridDim.x * threadIdx.x) : (int)(gridDim.x * TPB) + atomicAdd(work_counter, 1);
       first_wave = false;
-      active = idx < B * n_starts;
-      if (active) {
-        begin_item(cfg, batch, B, idx, u_init, p, sl, s, ref);
-        fresh = true;
+      if constexpr (kAdaptive) {
+        pending = true;
       } else {
-        saw_empty = true;
+        active = idx < B * n_starts;
+        if (active) {
+          begin_item(cfg, batch, B, idx, u_init, p, sl, s, ref);
+          fresh = true;
+        } else {
+          saw_empty = true;
+        }
+      }
+    }
+    if constexpr (kAdaptive) {
+      if (pending) {
+        const int r = poll_ticket(aq, B, n_starts, idx);
+        if (r != kTicketPending) {
+          pending = false;
+          active = r >= 0;
+          if (active) {
+            idx = r;
+            begin_item(cfg, batch, B, idx, u_init, p, sl, s, ref);
+            fresh = true;
+          } else {
+            saw_empty = true;
+          }
+        }
       }
     }
     __syncwarp();
@@ -315,15 +403,26 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
       // the winner commits.  Same iterates, same iteration counts, same results -- fewer trips in the tail,
       // where ~40 % of the trips of the slow problems are rejections.
       const int n_active = __syncthreads_count(active && spec_j == 0);
-      if (n_active == 0) break;
-      if (!drained) drained = __syncthreads_or(saw_empty) != 0;     // every decision below is taken on barrier results only
+      // kAdaptive: a pending lane keeps the block alive, and compaction (which reassigns lanes and would drop its
+      // ticket) waits until no lane is pending -- once some lane saw the queue empty, pending lanes resolve next trip
+      bool settled;
+      if constexpr (kAdaptive) {
+        const bool any_pending = __syncthreads_or(pending) != 0;
+        if (n_active == 0 && !any_pending) break;
+        if (!drained) drained = __syncthreads_or(saw_empty) != 0;
+        settled = drained && !any_pending;
+      } else {
+        if (n_active == 0) break;
+        if (!drained) drained = __syncthreads_or(saw_empty) != 0;     // every decision below is taken on barrier results only
+        settled = drained;
+      }
       int k_new = 1;
-      if (kSpec && drained) {                                // largest power of two with n_active * k <= MPC_SPEC_LANES, at most MPC_SPEC_MAXK
+      if (kSpec && settled) {                                // largest power of two with n_active * k <= MPC_SPEC_LANES, at most MPC_SPEC_MAXK
         while (2 * k_new <= MPC_SPEC_MAXK && n_active * 2 * k_new <= MPC_SPEC_LANES) k_new *= 2;
       }
       if (k_new < spec_k) k_new = spec_k;
       const int warps_new = (n_active * k_new + 31) >> 5;
-      if (drained && n_active <= kCompactMax && (k_new > spec_k || (live_warps > 1 && 2 * warps_new <= live_warps))) {
+      if (settled && n_active <= kCompactMax && (k_new > spec_k || (live_warps > 1 && 2 * warps_new <= live_warps))) {
         const bool lead = active && spec_j == 0;
         const unsigned bal = __ballot_sync(full, lead);
         const int lane = threadIdx.x & 31;
@@ -372,7 +471,7 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
       }
       if (warp >= live_warps) continue;                      // parked: nothing to sweep, back to the barrier
     } else {
-      if (!__any_sync(full, active)) break;
+      if (!__any_sync(full, active || pending)) break;
     }
     float d1 = 0.f, d2 = 0.f, alpha = 1.f, Jn = 0.f, md = 0.f;
     bool ok = false;
@@ -422,7 +521,10 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
         solve_init_finish(s, Jc);
         fresh = false;
       } else if (s.done) {
-        if (spec_j == 0) finish_item(cfg, out, cand, n_starts, idx, sl, s);
+        if (spec_j == 0) {
+          finish_item(cfg, out, cand, n_starts, idx, sl, s);
+          if constexpr (kAdaptive) if (idx < B * n_starts) publish_base(aq, cand, B, n_starts, idx);
+        }
         active = false;
         spec_j = 0;
         need_fetch = !drained;                               // nothing left to fetch once a lane of the block saw the queue empty
@@ -454,12 +556,16 @@ struct SmemOptIn {
   }
 };
 
-template <int TPB> static cudaError_t launch_solve_tmem_t(const SolveLaunch& s, cudaStream_t stream) {
+template <int TPB, bool kAdaptive> static cudaError_t launch_solve_tmem_t(const SolveLaunch& s, cudaStream_t stream) {
   static SmemOptIn opt;
-  cudaError_t e = opt.ensure(k_solve_tmem<TPB>, s.smem_bytes);
+  cudaError_t e = opt.ensure(k_solve_tmem<TPB, kAdaptive>, s.smem_bytes);
   if (e != cudaSuccess) return e;
-  k_solve_tmem<TPB><<<s.grid, TPB, s.smem_bytes, stream>>>(s.cfg, s.batch, s.out, s.B, s.work_counter, s.u_init, s.n_starts, s.cand);
+  k_solve_tmem<TPB, kAdaptive><<<s.grid, TPB, s.smem_bytes, stream>>>(s.cfg, s.batch, s.out, s.B, s.work_counter, s.u_init,
+                                                                       s.n_starts, s.cand, s.aq);
   return cudaGetLastError();
+}
+template <int TPB> static cudaError_t launch_solve_tmem_t(const SolveLaunch& s, cudaStream_t stream) {
+  return s.aq.max_starts > 0 ? launch_solve_tmem_t<TPB, true>(s, stream) : launch_solve_tmem_t<TPB, false>(s, stream);
 }
 
 cudaError_t launch_solve_tmem(const SolveLaunch& s, cudaStream_t stream) {
@@ -475,13 +581,17 @@ cudaError_t launch_solve_tmem(const SolveLaunch& s, cudaStream_t stream) {
   }
 }
 
-template <int TPB> static cudaError_t launch_solve_t(const SolveLaunch& s, cudaStream_t stream) {
+template <int TPB, bool kAdaptive> static cudaError_t launch_solve_t(const SolveLaunch& s, cudaStream_t stream) {
   // handles with different horizon / obstacle counts share the kernel: raise the opt-in limit as needed
   static SmemOptIn opt;
-  cudaError_t e = opt.ensure(k_solve<TPB>, s.smem_bytes);
+  cudaError_t e = opt.ensure(k_solve<TPB, kAdaptive>, s.smem_bytes);
   if (e != cudaSuccess) return e;
-  k_solve<TPB><<<s.grid, TPB, s.smem_bytes, stream>>>(s.cfg, s.batch, s.out, s.B, s.work_counter, s.u_init, s.n_starts, s.cand);
+  k_solve<TPB, kAdaptive><<<s.grid, TPB, s.smem_bytes, stream>>>(s.cfg, s.batch, s.out, s.B, s.work_counter, s.u_init, s.n_starts,
+                                                                  s.cand, s.aq);
   return cudaGetLastError();
+}
+template <int TPB> static cudaError_t launch_solve_t(const SolveLaunch& s, cudaStream_t stream) {
+  return s.aq.max_starts > 0 ? launch_solve_t<TPB, true>(s, stream) : launch_solve_t<TPB, false>(s, stream);
 }
 
 cudaError_t launch_solve(const SolveLaunch& s, cudaStream_t stream) {
@@ -521,6 +631,42 @@ k_select(const int B, const int S, const int N, const SolveCand cand, const MpcS
 
 cudaError_t launch_select(const SolveLaunch& s, cudaStream_t stream) {
   k_select<<<(s.B + 255) / 256, 256, 0, stream>>>(s.B, s.n_starts, s.cfg.N, s.cand, s.out);
+  return cudaGetLastError();
+}
+
+// Adaptive portfolio: the same selection over starts 0..S0-1, plus S0..S-1 for the problems the solve kernel extended
+// (base_done[b] == S0 + 1).  start_cost [S][ld] (NaN for starts that did not run) and extended [B] are optional.
+__global__ void __launch_bounds__(256)
+k_select_adaptive(const int B, const int S0, const int N, const SolveCand cand, const MpcSolveOut out, const AdaptiveQueue aq,
+                  float* __restrict__ start_cost, uint8_t* __restrict__ extended, const int ld) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const bool ext = aq.base_done[b] > S0;
+  const int S = ext ? aq.max_starts : S0;
+  int best = 0, it = 0;
+  float Jb = 0.f;
+  for (int st = 0; st < S; ++st) {
+    const float J = cand.cost[(size_t)st * B + b];
+    it += cand.iters[(size_t)st * B + b];
+    if (st == 0 || J < Jb) { Jb = J; best = st; }
+    if (st > 0 && !(Jb == Jb) && J == J) { Jb = J; best = st; }
+    if (start_cost) start_cost[(size_t)st * ld + b] = J;
+  }
+  if (start_cost)
+    for (int st = S; st < aq.max_starts; ++st) start_cost[(size_t)st * ld + b] = __int_as_float(0x7fc00000);
+  if (extended) extended[b] = ext ? 1 : 0;
+  const size_t w = (size_t)best * B + b;
+  out.actions[2 * (size_t)b] = cand.u0[2 * w];
+  out.actions[2 * (size_t)b + 1] = cand.u0[2 * w + 1];
+  if (out.status) out.status[b] = cand.status[w];
+  if (out.iters) out.iters[b] = it;
+  if (out.cost) out.cost[b] = Jb;
+  if (out.U)
+    for (int k = 0; k < 2 * N; ++k) out.U[(size_t)b * 2 * N + k] = cand.U[w * 2 * N + k];
+}
+
+cudaError_t launch_select_adaptive(const SolveLaunch& s, cudaStream_t stream) {
+  k_select_adaptive<<<(s.B + 255) / 256, 256, 0, stream>>>(s.B, s.n_starts, s.cfg.N, s.cand, s.out, s.aq, s.start_cost, s.extended, s.ld);
   return cudaGetLastError();
 }
 
