@@ -9,6 +9,7 @@
 #include <vector>
 
 #include "mpc_internal.h"
+#include "ref_path.h"
 
 using namespace mpcb;
 
@@ -28,6 +29,8 @@ struct MpcHandle {
   int tpb_small = 0;              // TMEM kernel: largest block the per-launch choice may use (<= 256)
   bool tpb_forced = false;
   // device workspace
+  void* ref_block = nullptr;      // the path tables built from cfg.dt (RefTables), uploaded once by mpc_create
+  RefTables tables{};
   void* ws_block = nullptr;       // one allocation carved into the BatchWs arrays
   BatchWs ws{};
   int* work_counter = nullptr;
@@ -75,6 +78,9 @@ static int fail(MpcHandle* h, int code, const char* what, cudaError_t e = cudaSu
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// dt arrives as a float (0.1f); the reference's dt is the double 1 / policy_frequency (agents/base_agent.py:43)
+static double prep_dt(float dt) { return 1.0 / (double)(long long)(1.0 / (double)dt + 0.5); }
+
 extern "C" {
 
 MPC_API const char* mpc_last_error(const MpcHandle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
@@ -84,7 +90,7 @@ MPC_API int mpc_destroy(MpcHandle* h) {
   cudaSetDevice(h->device);
   for (auto e : h->ev_prepare) cudaEventDestroy(e);
   for (auto e : h->ev_solve) cudaEventDestroy(e);
-  cudaFree(h->ws_block); cudaFree(h->work_counter); cudaFree(h->sink); cudaFree(h->aq_block);
+  cudaFree(h->ref_block); cudaFree(h->ws_block); cudaFree(h->work_counter); cudaFree(h->sink); cudaFree(h->aq_block);
   cudaFree(h->cand.cost); cudaFree(h->cand.u0); cudaFree(h->cand.status); cudaFree(h->cand.iters); cudaFree(h->cand.U);
   cudaFree(h->d_obs); cudaFree(h->d_ref_speed); cudaFree(h->d_weights); cudaFree(h->d_reset);
   cudaFree(h->d_actions); cudaFree(h->d_status); cudaFree(h->d_iters); cudaFree(h->d_cost);
@@ -188,8 +194,34 @@ MPC_API int mpc_create(const MpcConfig* cfg, int device, int max_batch, MpcHandl
   if (bps < 1) bps = 1;
   if (h->use_tmem) bps = 1;                                 // the CTA owns all 512 TMEM columns of its SM
   h->grid = h->sm_count * bps;
-  CKC(upload_ref_table_solve());
-  CKC(upload_ref_table_prepare());
+  {   // the path is accumulated with v * dt steps (agents/base_agent.py:118-154): each handle holds its own table, so
+      // handles with different policy frequencies coexist in one process
+    double ref[kNRef][4], seg[kNRef - 1], xy[kNRef * 2];
+    float hsc[kNRef * kRefStride];
+    build_reference_path(prep_dt(cfg->dt), ref);
+    for (int j = 0; j < kNRef; ++j) {
+      xy[2 * j] = ref[j][0];
+      xy[2 * j + 1] = ref[j][1];
+      hsc[j * kRefStride + 0] = (float)ref[j][3];
+      hsc[j * kRefStride + 1] = (float)sin(ref[j][3]);
+      hsc[j * kRefStride + 2] = (float)cos(ref[j][3]);
+    }
+    for (int j = 0; j < kNRef - 1; ++j) {
+      double dx = ref[j + 1][0] - ref[j][0], dy = ref[j + 1][1] - ref[j][1];
+      volatile double xx = dx * dx, yy = dy * dy;       // volatile: no host-side FMA contraction (np.linalg.norm rounds each)
+      seg[j] = sqrt(xx + yy);
+    }
+    const size_t o_seg = sizeof(ref), o_xy = o_seg + sizeof(seg), o_hsc = o_xy + sizeof(xy);
+    CKC(cudaMalloc(&h->ref_block, o_hsc + sizeof(hsc)));
+    char* tb = (char*)h->ref_block;
+    CKC(cudaMemcpy(tb, ref, sizeof(ref), cudaMemcpyHostToDevice));
+    CKC(cudaMemcpy(tb + o_seg, seg, sizeof(seg), cudaMemcpyHostToDevice));
+    CKC(cudaMemcpy(tb + o_xy, xy, sizeof(xy), cudaMemcpyHostToDevice));
+    CKC(cudaMemcpy(tb + o_hsc, hsc, sizeof(hsc), cudaMemcpyHostToDevice));
+    h->tables.ref = (const double*)tb;
+    h->tables.seg = (const double*)(tb + o_seg);
+    h->tables.solve = RefTab<float>{(const float*)(tb + o_hsc), (const double*)(tb + o_xy)};
+  }
 
   // parsed-problem workspace
   const size_t B = (size_t)max_batch;
@@ -284,7 +316,7 @@ MPC_API int mpc_rollout_cost(MpcHandle* h, const MpcProblemBatch* batch, int B, 
   if (!U || !X_out || !cost6_out || !total_out) return fail(h, MPC_ERR_BAD_ARG, "mpc_rollout_cost: null output/input");
   if (B == 0) return MPC_OK;
   CK(h, cudaSetDevice(h->device));
-  CK(h, launch_rollout_cost(h->scfg, *batch, B, U, X_out, cost6_out, total_out, (cudaStream_t)stream));
+  CK(h, launch_rollout_cost(h->scfg, h->tables.solve, *batch, B, U, X_out, cost6_out, total_out, (cudaStream_t)stream));
   h->launches += 1;
   return MPC_OK;
 }
@@ -350,7 +382,7 @@ MPC_API int mpc_solve(MpcHandle* h, const MpcProblemBatch* batch, int B, const M
   CK(h, cudaMemsetAsync(h->work_counter, 0, sizeof(int), st));
   SolveLaunch s;
   if (B > h->max_batch && h->n_starts > 1) return fail(h, MPC_ERR_TOO_LARGE, "mpc_solve: B exceeds max_batch of mpc_create");
-  s.cfg = h->scfg; s.batch = *batch; s.out = *out; s.B = B; s.work_counter = h->work_counter;
+  s.cfg = h->scfg; s.tables = h->tables.solve; s.batch = *batch; s.out = *out; s.B = B; s.work_counter = h->work_counter;
   s.n_starts = h->n_starts; s.cand = h->cand;
   s.u_init = h->u_init;
   s.aq = AdaptiveQueue{};
@@ -384,8 +416,8 @@ static int prepare_range(MpcHandle* h, const float* obs, const float* ref_speed,
   p.ws = h->ws;
   p.B = B; p.first = first; p.count = count;
   p.V = h->cfg.vehicles_count; p.M = h->scfg.M; p.N = h->scfg.N;
-  // dt arrives as float (0.1f); the reference's dt is the double 1/policy_frequency
-  p.dt = 1.0 / (double)(long long)(1.0 / (double)h->cfg.dt + 0.5) ;
+  p.dt = prep_dt(h->cfg.dt);
+  p.ref = h->tables.ref; p.seg = h->tables.seg;
   p.w_speed = h->cfg.weight_speed; p.w_control = h->cfg.weight_control; p.w_diff = h->cfg.weight_input_diff;
   p.collision_check = h->cfg.collision_check;
   CK(h, launch_prepare(p, st));

@@ -24,8 +24,19 @@ struct BatchWs {
   float* obstacles;
 };
 
+// The handle's path tables (device memory, built by mpc_create from its dt, ref_path.h): the (85, 4) FP64 rows and the
+// segment lengths for the collision prediction, FP64 positions and a float (heading, sin h, cos h) table for the solver.
+// Kernels stage them into shared memory.
+struct RefTables {
+  const double* ref;           // [kNRef][4]  x, y, v, heading
+  const double* seg;           // [kNRef - 1] |ref[j+1] - ref[j]|
+  RefTab<float> solve;         // xy [kNRef][2] FP64, hsc [kNRef][kRefStride] float
+};
+
 struct PrepareParams {
   const float* obs;            // [B][V][8]
+  const double* ref;           // RefTables::ref
+  const double* seg;           // RefTables::seg
   const float* ref_speed;      // [B] or null (NaN = none)
   const float* weights;        // [B][3] or null
   const uint8_t* reset_mask;   // [B] or null
@@ -42,7 +53,6 @@ struct PrepareParams {
 // launches (defined in mpc_prepare.cu, compiled with -fmad=false so that FP64 results are
 // bit-identical to the numpy oracle's un-fused arithmetic)
 cudaError_t launch_prepare(const PrepareParams& p, cudaStream_t stream);
-cudaError_t upload_ref_table_prepare();
 
 // defined in mpc_solve.cu
 // Candidate results of the start portfolio: work item w = start * B + problem.  Filled by the solve kernels when
@@ -68,6 +78,7 @@ struct AdaptiveQueue {
 };
 struct SolveLaunch {
   SolverConfig cfg;
+  RefTab<float> tables;   // the handle's path tables (RefTables::solve), staged into shared memory by every block
   MpcProblemBatch batch;
   MpcSolveOut out;
   int B;                  // problems
@@ -85,9 +96,8 @@ struct SolveLaunch {
   int ld;                 // row stride of start_cost
 };
 cudaError_t launch_solve(const SolveLaunch& s, cudaStream_t stream);
-cudaError_t launch_rollout_cost(const SolverConfig& cfg, const MpcProblemBatch& batch, int B, const float* U,
-                                float* X_out, float* cost6, float* total, cudaStream_t stream);
-cudaError_t upload_ref_table_solve();
+cudaError_t launch_rollout_cost(const SolverConfig& cfg, const RefTab<float>& tables, const MpcProblemBatch& batch, int B,
+                                const float* U, float* X_out, float* cost6, float* total, cudaStream_t stream);
 cudaError_t launch_fma_peak(float* sink, int iters, int grid, int block, cudaStream_t stream);
 size_t solve_smem_bytes(int N, int M, int tpb);
 size_t solve_smem_bytes_tmem(int N, int M, int tpb);

@@ -16,8 +16,6 @@
 // with sub-warp shuffles, lane 0 of the group updates the latch and writes the solve descriptor.
 #include "mpc_internal.h"
 
-#include "ref_table.inc"
-
 namespace mpcb {
 
 constexpr int kPred = 30;            // PREDICTION_HORIZON, agents/pure_mpc.py:554
@@ -26,21 +24,6 @@ constexpr int kSafetyBuffer = 5;     // SAFETY_BUFFER_POINTS, agents/pure_mpc.py
 constexpr int kMemorySteps = 10;     // collision_memory_steps, agents/pure_mpc.py:39
 constexpr double kMaxAccPred = 3.5;  // Vehicle.max_acceleration, agents/utils.py:39
 constexpr double kPi = 3.141592653589793;
-
-__constant__ double c_refd[kNRef][4];     // x, y, v, heading
-__constant__ double c_seg[kNRef - 1];     // |ref[j+1] - ref[j]|
-
-cudaError_t upload_ref_table_prepare() {
-  cudaError_t e = cudaMemcpyToSymbol(c_refd, kRefPath, sizeof(kRefPath));
-  if (e != cudaSuccess) return e;
-  double seg[kNRef - 1];
-  for (int j = 0; j < kNRef - 1; ++j) {
-    double dx = kRefPath[j + 1][0] - kRefPath[j][0], dy = kRefPath[j + 1][1] - kRefPath[j][1];
-    volatile double xx = dx * dx, yy = dy * dy;     // volatile: no host-side FMA contraction either
-    seg[j] = sqrt(xx + yy);
-  }
-  return cudaMemcpyToSymbol(c_seg, seg, sizeof(seg));
-}
 
 __device__ __forceinline__ double norm2(double dx, double dy) { return sqrt(dx * dx + dy * dy); }
 // argmin over distances compares the squared norms: sqrt is monotone, so the first minimum is the same index
@@ -61,12 +44,12 @@ k_prepare(const PrepareParams P) {
   constexpr int PPB = 256 / LPP;                      // environments per block
   __shared__ double s_ex[PPB][kPred + 1];
   __shared__ double s_ey[PPB][kPred + 1];
-  // the path table is indexed per lane (ego_index + idx, strided argmin): divergent __constant__ reads are
-  // serialised per distinct address, shared memory is not
+  // the handle's path table (built from its dt) is indexed per lane (ego_index + idx, strided argmin): staged once per
+  // block into shared memory, where divergent reads cost nothing extra
   __shared__ double s_ref[kNRef][4];
   __shared__ double s_seg[kNRef - 1];
-  for (int i = threadIdx.x; i < kNRef * 4; i += blockDim.x) (&s_ref[0][0])[i] = (&c_refd[0][0])[i];
-  for (int i = threadIdx.x; i < kNRef - 1; i += blockDim.x) s_seg[i] = c_seg[i];
+  for (int i = threadIdx.x; i < kNRef * 4; i += blockDim.x) (&s_ref[0][0])[i] = __ldg(P.ref + i);
+  for (int i = threadIdx.x; i < kNRef - 1; i += blockDim.x) s_seg[i] = __ldg(P.seg + i);
   __syncthreads();
   const int g = threadIdx.x / LPP;                    // group inside the block
   const int l = threadIdx.x % LPP;                    // lane inside the group

@@ -22,41 +22,21 @@
 
 #include "mpc_internal.h"
 
-#include "ref_table.inc"
-
 namespace mpcb {
-
-__constant__ float c_hsc[kNRef * kRefStride];     // heading, sin h, cos h
-__constant__ double c_xy[kNRef * 2];               // path positions, FP64
-
-cudaError_t upload_ref_table_solve() {
-  float h[kNRef * kRefStride];
-  double xy[kNRef * 2];
-  for (int j = 0; j < kNRef; ++j) {
-    xy[2 * j] = kRefPath[j][0];
-    xy[2 * j + 1] = kRefPath[j][1];
-    h[j * kRefStride + 0] = (float)kRefPath[j][3];
-    h[j * kRefStride + 1] = (float)sin(kRefPath[j][3]);
-    h[j * kRefStride + 2] = (float)cos(kRefPath[j][3]);
-  }
-  cudaError_t e = cudaMemcpyToSymbol(c_hsc, h, sizeof(h));
-  if (e != cudaSuccess) return e;
-  return cudaMemcpyToSymbol(c_xy, xy, sizeof(xy));
-}
 
 constexpr int kTabFloats = kNRef * 2 * 2 + kNRef * kRefStride + 1;   // FP64 xy (as 2 floats each) + hsc, padded to even
 size_t solve_smem_bytes(int N, int M, int tpb) {
   return (size_t)(kTabFloats + slots_per_problem(N, M, true) * tpb) * sizeof(float);
 }
 
-// block-shared copy of the path tables at the head of dynamic shared memory
-__device__ __forceinline__ RefTab<float> stage_tables(float* smem) {
+// block-shared copy of the handle's path tables (device memory, built from its dt) at the head of dynamic shared memory
+__device__ __forceinline__ RefTab<float> stage_tables(float* smem, const RefTab<float>& src) {
   double* xy = reinterpret_cast<double*>(smem);
   float* hsc = smem + kNRef * 2 * 2;
 #pragma unroll 1
-  for (int i = threadIdx.x; i < kNRef * 2; i += blockDim.x) xy[i] = c_xy[i];
+  for (int i = threadIdx.x; i < kNRef * 2; i += blockDim.x) xy[i] = __ldg(src.xy + i);
 #pragma unroll 1
-  for (int i = threadIdx.x; i < kNRef * kRefStride; i += blockDim.x) hsc[i] = c_hsc[i];
+  for (int i = threadIdx.x; i < kNRef * kRefStride; i += blockDim.x) hsc[i] = __ldg(src.hsc + i);
   __syncthreads();
   return RefTab<float>{hsc, xy};
 }
@@ -208,9 +188,9 @@ __device__ __forceinline__ void publish_base(const AdaptiveQueue& aq, const Solv
 template <int TPB, bool kAdaptive>
 __global__ void __launch_bounds__(TPB, 1)
 k_solve(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut out, const int B, int* __restrict__ work_counter,
-        const float* __restrict__ u_init, const int n_starts, const SolveCand cand, const AdaptiveQueue aq) {
+        const float* __restrict__ u_init, const int n_starts, const SolveCand cand, const AdaptiveQueue aq, const RefTab<float> tables) {
   extern __shared__ __align__(16) float smem[];
-  const RefTab<float> ref = stage_tables(smem);
+  const RefTab<float> ref = stage_tables(smem, tables);
   using SL = Slots<float, true, TPB>;
   const SL sl{smem + kTabFloats + threadIdx.x, TPB, cfg.N, cfg.M};
   const unsigned full = 0xffffffffu;
@@ -316,7 +296,8 @@ bool tmem_layout_fits(int N, int tpb) {
 template <int TPB, bool kAdaptive>
 __global__ void __launch_bounds__(TPB, 1)
 k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut out, const int B, int* __restrict__ work_counter,
-             const float* __restrict__ u_init, const int n_starts, const SolveCand cand, const AdaptiveQueue aq) {
+             const float* __restrict__ u_init, const int n_starts, const SolveCand cand, const AdaptiveQueue aq,
+             const RefTab<float> tables) {
   extern __shared__ __align__(16) float smem[];
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + kTabFloats);
   const int warp = threadIdx.x >> 5;
@@ -326,7 +307,7 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
   }
   asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
-  const RefTab<float> ref = stage_tables(smem);            // contains the __syncthreads()
+  const RefTab<float> ref = stage_tables(smem, tables);    // contains the __syncthreads()
   asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
   const uint32_t tmem_base = *s_tmem;
   using SL = SlotsTmem<TPB>;
@@ -561,7 +542,7 @@ template <int TPB, bool kAdaptive> static cudaError_t launch_solve_tmem_t(const 
   cudaError_t e = opt.ensure(k_solve_tmem<TPB, kAdaptive>, s.smem_bytes);
   if (e != cudaSuccess) return e;
   k_solve_tmem<TPB, kAdaptive><<<s.grid, TPB, s.smem_bytes, stream>>>(s.cfg, s.batch, s.out, s.B, s.work_counter, s.u_init,
-                                                                       s.n_starts, s.cand, s.aq);
+                                                                       s.n_starts, s.cand, s.aq, s.tables);
   return cudaGetLastError();
 }
 template <int TPB> static cudaError_t launch_solve_tmem_t(const SolveLaunch& s, cudaStream_t stream) {
@@ -587,7 +568,7 @@ template <int TPB, bool kAdaptive> static cudaError_t launch_solve_t(const Solve
   cudaError_t e = opt.ensure(k_solve<TPB, kAdaptive>, s.smem_bytes);
   if (e != cudaSuccess) return e;
   k_solve<TPB, kAdaptive><<<s.grid, TPB, s.smem_bytes, stream>>>(s.cfg, s.batch, s.out, s.B, s.work_counter, s.u_init, s.n_starts,
-                                                                  s.cand, s.aq);
+                                                                  s.cand, s.aq, s.tables);
   return cudaGetLastError();
 }
 template <int TPB> static cudaError_t launch_solve_t(const SolveLaunch& s, cudaStream_t stream) {
@@ -672,10 +653,10 @@ cudaError_t launch_select_adaptive(const SolveLaunch& s, cudaStream_t stream) {
 
 // ---- K1 parity entry: rollout + six cost components for given controls -----------------------
 __global__ void __launch_bounds__(64)
-k_rollout_cost(const SolverConfig cfg, const MpcProblemBatch batch, const int B, const float* __restrict__ U,
+k_rollout_cost(const SolverConfig cfg, const RefTab<float> tables, const MpcProblemBatch batch, const int B, const float* __restrict__ U,
                float* __restrict__ X_out, float* __restrict__ cost6, float* __restrict__ total) {
   extern __shared__ __align__(16) float smem[];
-  const RefTab<float> ref = stage_tables(smem);
+  const RefTab<float> ref = stage_tables(smem, tables);
   const Slots<float, true> sl{smem + kTabFloats + threadIdx.x, (int)blockDim.x, cfg.N, cfg.M};
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < B; i += gridDim.x * blockDim.x) {
     ProblemScalars<float> p;
@@ -700,8 +681,8 @@ k_rollout_cost(const SolverConfig cfg, const MpcProblemBatch batch, const int B,
   }
 }
 
-cudaError_t launch_rollout_cost(const SolverConfig& cfg, const MpcProblemBatch& batch, int B, const float* U,
-                                float* X_out, float* cost6, float* total, cudaStream_t stream) {
+cudaError_t launch_rollout_cost(const SolverConfig& cfg, const RefTab<float>& tables, const MpcProblemBatch& batch, int B,
+                                const float* U, float* X_out, float* cost6, float* total, cudaStream_t stream) {
   const int tpb = 64;
   size_t smem = solve_smem_bytes(cfg.N, cfg.M, tpb);
   cudaError_t e = cudaFuncSetAttribute(k_rollout_cost, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -709,7 +690,7 @@ cudaError_t launch_rollout_cost(const SolverConfig& cfg, const MpcProblemBatch& 
   int grid = (B + tpb - 1) / tpb;
   if (grid > 148 * 8) grid = 148 * 8;
   if (grid < 1) grid = 1;
-  k_rollout_cost<<<grid, tpb, smem, stream>>>(cfg, batch, B, U, X_out, cost6, total);
+  k_rollout_cost<<<grid, tpb, smem, stream>>>(cfg, tables, batch, B, U, X_out, cost6, total);
   return cudaGetLastError();
 }
 

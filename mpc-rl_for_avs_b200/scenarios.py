@@ -37,7 +37,7 @@ _LANE_HEADING = np.array([-math.pi / 2, 0.0, math.pi / 2, math.pi])
 
 
 def make_scenarios(batch: int, n_obstacles: int = 8, seed: int = 1234, vehicles_count: Optional[int] = None,
-                   ref_speed_fraction: float = 0.5, v_max: float = 12.0, same_lane_frac: float = 0.0
+                   ref_speed_fraction: float = 0.5, v_max: float = 12.0, same_lane_frac: float = 0.0, dt: float = 0.1
                    ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
     """Returns (obs [B,V,8] f32, ref_speed [B,1] f32, has_ref_speed [B] bool) on the CPU.
 
@@ -50,13 +50,15 @@ def make_scenarios(batch: int, n_obstacles: int = 8, seed: int = 1234, vehicles_
     centre x = 2.0 with heading -pi/2 (highway-env spawns on the lane centre, which is the reference path's own x) --
     the collinear / LineString branch of the reference's collision check (agents/pure_mpc.py:615-633).  Drawn from a
     separate stream so the default scenes do not change.
+    `dt` (the policy step, 1 / policy_frequency): the ego is placed on `reference_path(dt)`, the path an agent with that
+    policy frequency follows; the random draws do not depend on it.
     """
     g = torch.Generator(device="cpu")
     g.manual_seed(int(seed))
     V = vehicles_count if vehicles_count is not None else n_obstacles + 1
     if V < n_obstacles + 1:
         raise ValueError("vehicles_count must be >= n_obstacles + 1")
-    ref = reference_path()
+    ref = reference_path(dt)
     B, M = int(batch), int(n_obstacles)
 
     def randn(*s):

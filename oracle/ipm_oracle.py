@@ -41,17 +41,15 @@ from scipy.linalg import ldl
 import mpc_oracle as orc
 from mpc_oracle import Problem, Solution, N_REF, WHEELBASE, REAR_RATIO
 
-_REF = orc.reference_states()
-
-
 # ----------------------------------------------------------------------------------------
 # NLP functions of the literal formulation
 # ----------------------------------------------------------------------------------------
 class LiteralNLP:
     """f, grad f, g, Jacobian, Lagrangian Hessian of agents/pure_mpc.py:128-280 for one Problem."""
 
-    def __init__(self, prob: Problem, ref: np.ndarray = _REF):
+    def __init__(self, prob: Problem):
         self.p = prob
+        ref = prob.ref
         N = prob.N
         self.N, self.dt = N, prob.dt
         self.nx = 4 * (N + 1)
@@ -649,7 +647,7 @@ def path_following_controls(prob: Problem, mode: str = "ref", look: int = 1, sla
     `slalom`: from the first stage whose reference row is the frozen last row of the path (k >= 84 - ego_index) the
     steering alternates full right / full left every stage -- the shape of the optima past the end of the path.
     The device solver's path-following starts (mpc_core.cuh: apply_start) follow the same recipe in FP32."""
-    ref = orc.reference_states(prob.dt)
+    ref = prob.ref
     sb_max = math.sin(math.atan(orc.REAR_RATIO * math.tan(orc.DELTA_MAX)))
     U = np.zeros((prob.N, 2))
     s = np.asarray(prob.s0, dtype=np.float64).copy()
@@ -694,7 +692,7 @@ def best_known_optimum(prob: Problem, cpu_starts: int = 4, path_starts: int = 2)
         sk = orc.solve_nlp(prob, U0=path_following_controls(prob, mode))
         Uk, ck, okk = polish_fixed_point(prob, sk.U)
         cands.append((f"slsqp_path_{mode}", Uk, ck, okk))
-    if path_starts and prob.ego_index + prob.N > orc.reference_states(prob.dt).shape[0] - 1:
+    if path_starts and prob.ego_index + prob.N > prob.ref.shape[0] - 1:
         sk = orc.solve_nlp(prob, U0=path_following_controls(prob, "ref", 1, slalom=True))
         Uk, ck, okk = polish_fixed_point(prob, sk.U)
         cands.append(("slsqp_slalom", Uk, ck, okk))

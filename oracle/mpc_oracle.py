@@ -38,6 +38,7 @@ State order [x, y, theta, v], control order [a, delta]  (agents/pure_mpc.py:88-8
 """
 from __future__ import annotations
 
+import functools
 import math
 from dataclasses import dataclass, field
 from typing import List, Optional, Sequence, Tuple
@@ -88,6 +89,15 @@ def reference_states(dt: float = 0.1) -> np.ndarray:
         y += 0
         rows.append((x, y, v, h))
     return np.array(rows, dtype=np.float64)
+
+
+@functools.lru_cache(maxsize=None)
+def path_table(dt: float = 0.1) -> np.ndarray:
+    """reference_states(dt), computed once per dt and read-only: the table every function below takes from
+    `Problem.ref` or from its own dt."""
+    t = reference_states(dt)
+    t.setflags(write=False)
+    return t
 
 
 def normalize_angle(angle: float) -> float:
@@ -239,8 +249,10 @@ class Problem:
     literal_no_collision: bool = False             # A15: objective = control + input_diff only
     ref_v_final: float = 10.0                      # reference speed at row j(N) (final_state_cost only)
 
-
-_REF = reference_states()
+    @property
+    def ref(self) -> np.ndarray:
+        """The path table of this problem's time step: the reference accumulates its rows with v * dt steps."""
+        return path_table(self.dt)
 
 
 def obstacle_positions(others: np.ndarray, N: int, dt: float) -> np.ndarray:
@@ -257,11 +269,11 @@ def obstacle_positions(others: np.ndarray, N: int, dt: float) -> np.ndarray:
     return P
 
 
-def cost_components(X: np.ndarray, U: np.ndarray, prob: Problem, ref: np.ndarray = _REF) -> np.ndarray:
+def cost_components(X: np.ndarray, U: np.ndarray, prob: Problem) -> np.ndarray:
     """The six un-weighted components [state, control, final_state, input_diff, distance,
     collision] of the reference's `cost_fn` (agents/pure_mpc.py:128-202, 215-216; distance
     term as in agents/archive/pure_mpc.py:189-196; collision term pure_mpc.py:179-183)."""
-    N = prob.N
+    N, ref = prob.N, prob.ref
     j = np.minimum(prob.ego_index + np.arange(N), N_REF - 1)
     rx, ry, rh = ref[j, 0], ref[j, 1], ref[j, 3]
     dx, dy = X[:N, 0] - rx, X[:N, 1] - ry
@@ -298,9 +310,9 @@ def objective(U: np.ndarray, prob: Problem) -> float:
     return total_cost_from_components(cost_components(X, U, prob), prob)
 
 
-def objective_and_sens(Uflat: np.ndarray, prob: Problem, ref: np.ndarray = _REF):
+def objective_and_sens(Uflat: np.ndarray, prob: Problem):
     """f, grad f (2N,), X (N+1,4), S (N+1, 4, 2N) with S[k] = d X[k] / d U."""
-    N, dt = prob.N, prob.dt
+    N, dt, ref = prob.N, prob.dt, prob.ref
     U = Uflat.reshape(N, 2)
     X = np.empty((N + 1, 4))
     S = np.zeros((N + 1, 4, 2 * N))
@@ -310,7 +322,7 @@ def objective_and_sens(Uflat: np.ndarray, prob: Problem, ref: np.ndarray = _REF)
         X[k + 1] = step(X[k], U[k], dt)
         S[k + 1] = A @ S[k]
         S[k + 1][:, 2 * k:2 * k + 2] += B
-    c = cost_components(X, U, prob, ref)
+    c = cost_components(X, U, prob)
     f = total_cost_from_components(c, prob)
     g = np.zeros(2 * N)
     # control + input-difference parts
@@ -482,7 +494,8 @@ def solve_nlp_multiple_shooting(prob: Problem, maxiter: int = 800, ftol: float =
         gU[:-1] -= prob.w_input_diff * 0.02 * dU
         if not prob.literal_no_collision:
             j = np.minimum(prob.ego_index + np.arange(N), N_REF - 1)
-            rx, ry, rh = _REF[j, 0], _REF[j, 1], _REF[j, 3]
+            ref = prob.ref
+            rx, ry, rh = ref[j, 0], ref[j, 1], ref[j, 3]
             sh, ch = np.sin(rh), np.cos(rh)
             dx, dy = X[:N, 0] - rx, X[:N, 1] - ry
             perp = dx * sh - dy * ch
@@ -541,11 +554,12 @@ def solve_nlp_multiple_shooting(prob: Problem, maxiter: int = 800, ftol: float =
 # collision prediction (agents/pure_mpc.py:459-676)
 # ----------------------------------------------------------------------------------------
 def predict_ego_polyline(pos: np.ndarray, speed: float, start_index: int, ref_speed: float,
-                         dt: float = 0.1, ref: np.ndarray = _REF) -> np.ndarray:
+                         dt: float = 0.1, ref: Optional[np.ndarray] = None) -> np.ndarray:
     """Path-following prediction of the ego (agents/pure_mpc.py:459-527): point 0 is the
     actual position; the speed ramps by 3.5*dt up to `ref_speed` (or snaps down to it);
     the travelled arc length is mapped onto the reference polyline from `start_index`
-    by a left searchsorted + linear interpolation; stops once past the path end."""
+    by a left searchsorted + linear interpolation; stops once past the path end.  `ref` defaults to the table of dt."""
+    ref = path_table(dt) if ref is None else ref
     pts = [np.array(pos, dtype=np.float64)]
     rp = ref[start_index:, :2]
     if rp.shape[0] < 2:
@@ -718,9 +732,10 @@ class CollisionResult:
 
 
 def detect_collisions(ego: np.ndarray, others: np.ndarray, dt: float = 0.1,
-                      ref: np.ndarray = _REF) -> CollisionResult:
+                      ref: Optional[np.ndarray] = None) -> CollisionResult:
     """The detection body of `_check_collision` (agents/pure_mpc.py:565-661), without the
-    latch.  `ego` = (x, y, theta, v); `others` rows (x, y, speed, heading)."""
+    latch.  `ego` = (x, y, theta, v); `others` rows (x, y, speed, heading).  `ref` defaults to the table of dt."""
+    ref = path_table(dt) if ref is None else ref
     ref_xy = ref[:, :2]
     ego_index = nearest_index(ego[:2], ref_xy)
     E = predict_ego_polyline(ego[:2], ego[3], ego_index, ref[ego_index, 2], dt, ref)
@@ -749,9 +764,10 @@ def detect_collisions(ego: np.ndarray, others: np.ndarray, dt: float = 0.1,
 def regenerate_ref_speed(ego_index: int, v_ego: float, is_collide: bool,
                          conflict_index: Sequence[Optional[int]],
                          ref_speed_override: Optional[float] = None,
-                         ref: np.ndarray = _REF) -> Tuple[np.ndarray, Optional[int]]:
+                         ref: Optional[np.ndarray] = None) -> Tuple[np.ndarray, Optional[int]]:
     """Speed column of `update_reference_states` (agents/pure_mpc.py:678-724).
-    Returns (ref_speed[85], stop_index or None)."""
+    Returns (ref_speed[85], stop_index or None).  Only the speed column of `ref` is read (10 at every dt)."""
+    ref = path_table() if ref is None else ref
     col = ref[:, 2].copy()
     if ref_speed_override is not None:                         # :683-688, takes precedence
         col[:] = min(max(float(ref_speed_override), 0.0), 30.0)
@@ -788,7 +804,7 @@ class OraclePureMPCAgent:
         self.w_distance, self.w_collision = weight_distance, weight_collision
         self.collision_check = collision_check
         self.literal_no_collision = literal_no_collision
-        self.ref = reference_states(dt)
+        self.ref = path_table(dt)
         self.collision_memory = 0
         self.memorized_conflict_indices: Optional[list] = None
         self.conflict_index: list = []

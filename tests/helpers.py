@@ -21,11 +21,11 @@ REF = orc.reference_states()
 
 
 # ----------------------------------------------------------------------------- problems
-def problems_from_obs(obs, ref_speed=None, has_ref_speed=None, w_distance=0.0, collision_check=False, N=20):
+def problems_from_obs(obs, ref_speed=None, has_ref_speed=None, w_distance=0.0, collision_check=False, N=20, dt=0.1):
     """One fresh oracle agent per observation (cleared latch): parse -> [collision] -> Problem."""
     probs, agents = [], []
     for i in range(obs.shape[0]):
-        ag = orc.OraclePureMPCAgent(horizon=N, vehicles_count=obs.shape[1], weight_distance=w_distance,
+        ag = orc.OraclePureMPCAgent(horizon=N, dt=dt, vehicles_count=obs.shape[1], weight_distance=w_distance,
                                     collision_check=collision_check)
         parsed = orc.parse_obs(obs[i], obs.shape[1])
         if collision_check:
@@ -36,6 +36,24 @@ def problems_from_obs(obs, ref_speed=None, has_ref_speed=None, w_distance=0.0, c
         probs.append(ag.build_problem(parsed, None, r))
         agents.append(ag)
     return probs, agents
+
+
+def config_scenes(B, N, M, dt, seed, w_distance=None, same_lane_frac=0.0):
+    """Seeded scenes of a configuration off the shipped one: B environments with M other vehicles, the ego placed on the
+    path of time step dt (scenarios.make_scenarios), and their oracle problems of horizon N (collision logic on,
+    distance term 10 when there is traffic).  Returns (obs [B, M+1, 8] f32, ref_speed [B] f32 with NaN where the scene
+    has none, probs)."""
+    import mpc_rl_for_avs_b200 as pkg
+    wd = (10.0 if M > 0 else 0.0) if w_distance is None else w_distance
+    obs, rs, has = pkg.make_scenarios(B, M, seed=seed, dt=dt, same_lane_frac=same_lane_frac)
+    obs, rs, has = obs.numpy(), rs.numpy(), has.numpy()
+    probs, _ = problems_from_obs(obs, rs, has, w_distance=wd, collision_check=True, N=N, dt=dt)
+    return obs, np.where(has, rs[:, 0], np.nan).astype(np.float32), probs
+
+
+# (N, M, dt) points of the rollout / cost parity tests: the smallest horizons, a vehicle count on each prepare kernel,
+# horizons that clamp at the path's last row, and four policy frequencies
+ROLLOUT_CONFIGS = [(2, 1, 0.1), (3, 0, 0.2), (16, 9, 0.1), (33, 16, 0.05), (64, 8, 0.1), (20, 8, 1 / 15)]
 
 
 def ref_speed_descriptor(rv, rv_final=None):
@@ -101,6 +119,17 @@ class HsBatch(C.Structure):
                 ("is_collide", _P(C.c_ubyte)), ("n_obs", _P(C.c_int)), ("obstacles", _P(C.c_float))]
 
 
+def policy_dt(dt):
+    """The double 1 / policy_frequency for a (float32) time step: the dt of the reference's path table and collision
+    prediction (agents/base_agent.py:43), as the library derives it from MpcConfig.dt."""
+    return 1.0 / round(1.0 / float(dt))
+
+
+def cfg_ref(cfg):
+    """The oracle's path table for a harness config: the hostsim gets the table of the config's dt."""
+    return np.ascontiguousarray(orc.path_table(policy_dt(cfg.dt)))
+
+
 def hs_config(N=20, M=8, dt=0.1, w_distance=0.0, w_collision=0.0, literal=0, max_iter=60, tol_step=1e-4, reg_min=1e-2, stall_tol=0.0, kink_tol=1e-7):
     return HsConfig(N=N, M=M, dt=dt, w_distance=w_distance, w_collision=w_collision, literal_no_collision=literal,
                     max_iter=max_iter, tol_step=tol_step, reg_min=reg_min, stall_tol=stall_tol, kink_tol=kink_tol)
@@ -110,13 +139,20 @@ def load_hostsim():
     """Builds (if stale) and loads tests/hostsim/libhostsim.so -- the kernel's device functions
     compiled for the CPU.  Test infrastructure only; the product never loads it."""
     src = os.path.join(ROOT, "tests", "hostsim", "hostsim.cpp")
-    core = os.path.join(ROOT, "mpc-rl_for_avs_b200", "csrc", "mpc_core.cuh")
+    deps = [src] + [os.path.join(ROOT, "mpc-rl_for_avs_b200", "csrc", f) for f in ("mpc_core.cuh", "ref_path.h")]
     so = os.path.join(ROOT, "tests", "hostsim", "libhostsim.so")
-    if not os.path.exists(so) or os.path.getmtime(so) < max(os.path.getmtime(src), os.path.getmtime(core)):
+    if not os.path.exists(so) or os.path.getmtime(so) < max(os.path.getmtime(f) for f in deps):
         subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", so, src])
     lib = C.CDLL(so)
     assert lib.hs_sizeof_config() == C.sizeof(HsConfig)
     return lib
+
+
+def hostsim_reference_path(lib, dt):
+    """The library's own path-table generator (csrc/ref_path.h, what mpc_create uploads) at the double time step dt."""
+    out = np.zeros((orc.N_REF, 4), np.float64)
+    lib.hs_reference_path(C.c_double(dt), out.ctypes.data_as(_P(C.c_double)))
+    return out
 
 
 def _as_struct(d):
@@ -133,7 +169,7 @@ def hostsim_solve(lib, d, cfg, use_double=False):
     cost = np.zeros(B, np.float32); U = np.zeros((B, cfg.N, 2), np.float32); outer = np.zeros(B, np.int32)
     b = _as_struct(d)
     f = lambda a, t: a.ctypes.data_as(_P(t))  # noqa: E731
-    lib.hs_solve(C.byref(cfg), REF.ctypes.data_as(_P(C.c_double)), C.byref(b), B, int(use_double), f(act, C.c_float),
+    lib.hs_solve(C.byref(cfg), cfg_ref(cfg).ctypes.data_as(_P(C.c_double)), C.byref(b), B, int(use_double), f(act, C.c_float),
                  f(st, C.c_int), f(it, C.c_int), f(cost, C.c_float), f(U, C.c_float), f(outer, C.c_int))
     return dict(actions=act, status=st, iters=it, cost=cost, U=U)
 
@@ -147,7 +183,7 @@ def hostsim_solve_init(lib, d, cfg, U0=None, use_double=False, n_starts=1):
     cost = np.zeros(B, np.float32); U = np.zeros((B, cfg.N, 2), np.float32)
     b = _as_struct(d)
     f = lambda a, t: a.ctypes.data_as(_P(t))  # noqa: E731
-    lib.hs_solve_init(C.byref(cfg), REF.ctypes.data_as(_P(C.c_double)), C.byref(b), B, int(use_double),
+    lib.hs_solve_init(C.byref(cfg), cfg_ref(cfg).ctypes.data_as(_P(C.c_double)), C.byref(b), B, int(use_double),
                       None if U0 is None else f(U0, C.c_float), int(n_starts), f(act, C.c_float), f(st, C.c_int), f(it, C.c_int), f(cost, C.c_float), f(U, C.c_float))
     return dict(actions=act, status=st, iters=it, cost=cost, U=U)
 
@@ -158,7 +194,7 @@ def hostsim_rollout_cost(lib, d, cfg, U, use_double=False):
     X = np.zeros((B, cfg.N + 1, 4), np.float32); c6 = np.zeros((B, 6), np.float32); tot = np.zeros(B, np.float32)
     b = _as_struct(d)
     f = lambda a, t: a.ctypes.data_as(_P(t))  # noqa: E731
-    lib.hs_rollout_cost(C.byref(cfg), REF.ctypes.data_as(_P(C.c_double)), C.byref(b), B, int(use_double),
+    lib.hs_rollout_cost(C.byref(cfg), cfg_ref(cfg).ctypes.data_as(_P(C.c_double)), C.byref(b), B, int(use_double),
                         f(U, C.c_float), f(X, C.c_float), f(c6, C.c_float), f(tot, C.c_float))
     return X, c6, tot
 
@@ -204,6 +240,35 @@ def distance_conditioning(prob, U, pos_err=2e-6, disc_band=1e-4):
     d = np.hypot(X[:prob.N, None, 0] - P[:, :, 0], X[:prob.N, None, 1] - P[:, :, 1])
     c = np.where(d < 1.0, 1000.0, 100.0)
     return bool(np.any(np.abs(d - 1.0) < disc_band)), float(np.sum(2.0 * c / (d + 1e-6) ** 3) * pos_err)
+
+
+def check_rollout_cost(probs, U, X, c6, tot):
+    """Rollout states X [B, N+1, 4], the six cost components c6 [B, 6] and the total tot [B] of the float32 controls U
+    against the oracle's FP64 evaluation of the same float32 inputs: 1e-5 relative with a floor of 1, and the
+    conditioning of the distance term near contact.  A position floor is also the path length travelled: FP32 rounds the
+    heading to ~2e-7 rad, which moves the position by that much per metre driven (at H = 64, 1e-5 of 46 m on a
+    coordinate of 2 m).  The components may also differ by what that state error explains: the FP64 components at the
+    device's own states minus those at the oracle's (at H = 64 the tracking terms see 1e-5 m over 64 stages); a wrong
+    cost formula shows up against both."""
+    for i in range(len(probs)):
+        p = problem_f32(probs[i])
+        Xo = orc.rollout(p.s0, U[i].astype(np.float64), p.dt)
+        co = orc.cost_components(Xo, U[i].astype(np.float64), p)
+        scale = np.maximum(np.abs(Xo), 1.0)
+        scale[:, :2] = np.maximum(scale[:, :2], np.sum(np.hypot(np.diff(Xo[:, 0]), np.diff(Xo[:, 1]))))
+        assert np.max(np.abs(X[i] - Xo) / scale) <= 1e-5, i
+        # the distance term's conditioning at the position error actually seen (long horizons drift further than 2e-6 m)
+        near_disc, dist_tol = distance_conditioning(p, U[i], pos_err=max(2e-6, float(np.abs(X[i][:, :2] - Xo[:, :2]).max())))
+        if near_disc:
+            continue                                   # FP32 / FP64 may sit on different sides of the d = 1 jump
+        co_x = orc.cost_components(X[i].astype(np.float64), U[i].astype(np.float64), p)   # at the device's states
+        tol = 1e-5 * np.maximum(np.abs(co), 1.0) + np.abs(co_x - co)
+        tol[4] += dist_tol                             # conditioning of 1/d^2 near contact
+        assert np.all(np.abs(c6[i] - co) <= tol), (i, c6[i], co)
+        to = orc.total_cost_from_components(co, p)
+        to_x = orc.total_cost_from_components(co_x, p)
+        assert abs(tot[i] - to) <= 1e-5 * max(abs(to), 1.0) + abs(to_x - to) + p.w_distance * dist_tol, (i, tot[i], to)
+
 
 
 # ----------------------------------------------------------------------------- solve parity statistics

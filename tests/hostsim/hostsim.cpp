@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "../../mpc-rl_for_avs_b200/csrc/mpc_core.cuh"
+#include "../../mpc-rl_for_avs_b200/csrc/ref_path.h"
 
 using namespace mpcb;
 
@@ -160,6 +161,9 @@ int hs_rollout_cost(const SolverConfig* cfg, const double* ref85x4, const HsBatc
 }
 
 int hs_sizeof_config() { return (int)sizeof(SolverConfig); }
+
+// the library's path-table generator (what mpc_create builds from the handle's dt): out [85][4]
+void hs_reference_path(double dt, double* out) { build_reference_path(dt, reinterpret_cast<double (*)[4]>(out)); }
 }
 
 // debugging aid: model-vs-actual merit along the DDP step from a given nominal U

@@ -57,7 +57,7 @@ def hostsim_starts(lib, d, cfg, n_starts):
     it = np.zeros((n_starts, B), np.int32); u0 = np.zeros((n_starts, B, 2), np.float32)
     b = helpers._as_struct(d)
     f = lambda a, t: a.ctypes.data_as(P(t))  # noqa: E731
-    lib.hs_solve_starts(C.byref(cfg), helpers.REF.ctypes.data_as(P(C.c_double)), C.byref(b), B, n_starts, f(cost, C.c_float),
+    lib.hs_solve_starts(C.byref(cfg), helpers.cfg_ref(cfg).ctypes.data_as(P(C.c_double)), C.byref(b), B, n_starts, f(cost, C.c_float),
                         f(st, C.c_int), f(it, C.c_int), f(u0, C.c_float))
     return cost, st, it, u0
 

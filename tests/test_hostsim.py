@@ -19,30 +19,42 @@ def _problems(g):
     return probs
 
 
-@pytest.mark.parametrize("name,M,wd", [("golden_track", 0, 0.0), ("golden_coll", 8, 10.0)])
-@pytest.mark.parametrize("use_double", [False, True])
-def test_rollout_cost_matches_oracle(hostsim, name, M, wd, use_double):
-    g = helpers.load_golden(name)
-    probs = _problems(g)[:64]
-    d = {k: (v[..., :64] if v.ndim > 1 else v[:64]) for k, v in _golden_batch(g).items()}
-    d = {k: np.ascontiguousarray(v) for k, v in d.items()}
+def _rollout_inputs(hostsim, name, N, M, wd, dt, B=64):
+    """(problems, SoA batch, controls): a golden set, or seeded scenes of the configuration (N, M, dt).  The controls are
+    random, and near-optimal for the first quarter (the golden optimum, or the host build's own solution): the cancellation
+    regime near an optimum."""
     rng = np.random.default_rng(3)
-    U = np.stack([rng.uniform(-5, 5, (64, 20)), rng.uniform(-1.0, 1.0, (64, 20))], axis=-1).astype(np.float32)
-    U[:16] = g["oracle_U"][:16].astype(np.float32)
-    X, c6, tot = helpers.hostsim_rollout_cost(hostsim, d, helpers.hs_config(M=M, w_distance=wd), U, use_double)
-    for i in range(64):
-        p = helpers.problem_f32(probs[i])
-        Xo = orc.rollout(p.s0, U[i].astype(np.float64), p.dt)
-        co = orc.cost_components(Xo, U[i].astype(np.float64), p)
-        assert np.max(np.abs(X[i] - Xo) / np.maximum(np.abs(Xo), 1.0)) <= 1e-5, i
-        near_disc, dist_tol = helpers.distance_conditioning(p, U[i])
-        if near_disc:
-            continue
-        tol = 1e-5 * np.maximum(np.abs(co), 1.0)
-        tol[4] += dist_tol
-        assert np.all(np.abs(c6[i] - co) <= tol), (i, c6[i], co)
-        to = orc.total_cost_from_components(co, p)
-        assert abs(tot[i] - to) <= 1e-5 * max(abs(to), 1.0) + p.w_distance * dist_tol
+    U = np.stack([rng.uniform(-5, 5, (B, N)), rng.uniform(-1.0, 1.0, (B, N))], axis=-1).astype(np.float32)
+    if name.startswith("golden"):
+        g = helpers.load_golden(name)
+        probs = _problems(g)[:B]
+        d = {k: np.ascontiguousarray(v[..., :B] if v.ndim > 1 else v[:B]) for k, v in _golden_batch(g).items()}
+        U[:B // 4] = g["oracle_U"][:B // 4].astype(np.float32)
+    else:
+        _, _, probs = helpers.config_scenes(B, N, M, dt, seed=11 + N + M)
+        d = helpers.batch_from_problems(probs, M)
+        r = helpers.hostsim_solve(hostsim, {k: np.ascontiguousarray(v[..., :B // 4]) for k, v in d.items()},
+                                  helpers.hs_config(N=N, M=M, dt=dt, w_distance=wd))
+        U[:B // 4] = r["U"]
+    return probs, d, U
+
+
+ROLLOUT_CASES = [pytest.param("golden_track", 20, 0, 0.0, 0.1, id="golden_track-0-0.0"),
+                 pytest.param("golden_coll", 20, 8, 10.0, 0.1, id="golden_coll-8-10.0")] + [
+    pytest.param("scenes", N, M, 10.0 if M else 0.0, dt, id=f"N{N}-M{M}-f{round(1 / dt)}") for N, M, dt in helpers.ROLLOUT_CONFIGS]
+
+
+@pytest.mark.parametrize("name,N,M,wd,dt", ROLLOUT_CASES)
+@pytest.mark.parametrize("use_double", [False, True])
+def test_rollout_cost_matches_oracle(hostsim, name, N, M, wd, dt, use_double):
+    """Rollout and cost components of the host build against the oracle: the golden sets (H=20, dt=0.1) and the
+    configurations of helpers.ROLLOUT_CONFIGS (horizons 2..64, 0..16 other vehicles, policy frequencies 5..20; with
+    N >= 16 most horizons run past the path's last row, where the reference row and the final-state row clamp)."""
+    probs, d, U = _rollout_inputs(hostsim, name, N, M, wd, dt)
+    X, c6, tot = helpers.hostsim_rollout_cost(hostsim, d, helpers.hs_config(N=N, M=M, dt=dt, w_distance=wd), U, use_double)
+    if name == "scenes" and N > 20:
+        assert sum(p.ego_index + N > 84 for p in probs) >= len(probs) // 8
+    helpers.check_rollout_cost(probs, U, X, c6, tot)
 
 
 @pytest.mark.parametrize("name,M,wd", [("golden_track", 0, 0.0), ("golden_coll", 8, 10.0), ("golden_holdout", 8, 10.0),
@@ -109,5 +121,19 @@ def test_horizon16_solver_logic(hostsim):
     conv = r["status"] == 0
     assert conv.mean() >= 0.8
     for i in np.nonzero(conv)[0][:12]:
+        ok, du0, gain = helpers.oracle_warm_confirms(probs[i], r["U"][i])
+        assert ok, (i, du0, gain)
+
+
+def test_solver_logic_at_policy_frequency_5(hostsim):
+    """dt = 0.2: the problems are built on the path table of that dt (1 m -> 2 m row spacing).  Every status-0 solution
+    of a sample of 16 is confirmed by the oracle started at it."""
+    B, N, M, dt = 48, 20, 8, 0.2
+    _, _, probs = helpers.config_scenes(B, N, M, dt, seed=5)
+    r = helpers.hostsim_solve_init(hostsim, helpers.batch_from_problems(probs, M), helpers.hs_config(N=N, M=M, dt=dt, w_distance=10.0),
+                                   n_starts=4)
+    conv = r["status"] == 0
+    assert conv.mean() >= 0.7, conv.mean()
+    for i in np.nonzero(conv)[0][:16]:
         ok, du0, gain = helpers.oracle_warm_confirms(probs[i], r["U"][i])
         assert ok, (i, du0, gain)

@@ -10,20 +10,17 @@ import helpers
 from helpers import orc
 
 
-def test_reference_path_known_answers():
+def test_reference_path_known_answers_and_the_library_generator(hostsim):
     r = orc.reference_states()
     assert r.shape == (85, 4)
     assert np.allclose(r[0], (2, 49, 10, -np.pi / 2))
     assert np.allclose(r[39], (2, 10, 10, -np.pi / 2))
     assert np.allclose(r[59], (-11.22584979, -2.22584979, 10, -np.pi), atol=1e-8)
     assert np.allclose(r[84], (-36.22584979, -2.22584979, 10, -np.pi), atol=1e-8)
-    # the product's table generator and the generated CUDA include are bit-identical to the oracle's
+    # the product's python table and the library's C++ generator (csrc/ref_path.h) are bit-identical to the oracle's
     import mpc_rl_for_avs_b200 as pkg
     assert np.array_equal(pkg.reference_path(), r)
-    import os
-    inc = open(os.path.join(helpers.ROOT, "mpc-rl_for_avs_b200", "csrc", "ref_table.inc")).read()
-    vals = [float.fromhex(t.strip(" {},")) for line in inc.splitlines() if line.strip().startswith("{") for t in line.split(",") if "p" in t]
-    assert np.array_equal(np.array(vals).reshape(85, 4), r)
+    assert np.array_equal(helpers.hostsim_reference_path(hostsim, 0.1), r)
 
 
 def _mk(s0, **kw):
