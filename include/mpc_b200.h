@@ -196,6 +196,27 @@ MPC_API int mpc_predict_host(MpcHandle* h, const float* obs_host, const float* r
                      float* actions_host, int32_t* status_host, uint8_t* is_collide_host,
                      const MpcCollisionOut* col_host, int64_t* h2d_bytes, int64_t* d2h_bytes);
 
+/* Optimality certificate of controls U [B][N][2] (e.g. MpcSolveOut.U of a solve), in FP64, one value per problem:
+ * exactly the oracle's first-order test (oracle/mpc_oracle.py kkt_residual).  With g = grad_U J (the objective the solver
+ * minimises, rolled out without clamping) and the active set = every control bound and every theta / v bound of nodes
+ * 1..N within act_tol of its limit, residual = min_{mu >= 0} || g - J_act^T mu ||_2, the distance of g from the cone of
+ * the active constraint gradients (unique even where the multipliers are not).  A residual small against 1 + |J| certifies
+ * a first-order local optimum of the reference NLP; IPOPT reports the same quantity through solver.stats()
+ * (agents/pure_mpc.py:303).  Any pointer of MpcKktOut except residual may be NULL.  Non-finite controls or rollouts give
+ * a NaN residual.  Exact for every active-set size a horizon allows.
+ * batch == NULL certifies against the handle's workspace, i.e. the problems of the last mpc_prepare / mpc_predict(_host)
+ * call, whose B it must repeat.  act_tol must be >= 0 and not NaN.  No host synchronisation (capturable in a CUDA graph). */
+typedef struct MpcKktOut {
+  float* residual;            /* [B]  min_{mu >= 0} || g - J_act^T mu ||_2 */
+  float* grad_norm;           /* [B]  || g ||_2 */
+  float* violation;           /* [B]  largest violation of a control or node bound (0 = feasible) */
+  int32_t* n_active;          /* [B]  active constraint rows */
+  float* multipliers;         /* [B][N][4]  mu of a_k, mu of delta_k, nu of theta_{k+1}, nu of v_{k+1}: > 0 at an upper
+                               * bound, < 0 at a lower bound, 0 when inactive, so that g + sum mult * d(bounded)/dU = r */
+} MpcKktOut;
+MPC_API int mpc_kkt(MpcHandle* h, const MpcProblemBatch* batch, int B, const float* U, float act_tol, const MpcKktOut* out,
+                    void* stream);
+
 /* Measurement helpers */
 /* number of this library's kernel launches since mpc_create (bench.py's gpu_launches) */
 MPC_API int64_t mpc_launch_count(const MpcHandle* h);

@@ -67,10 +67,15 @@ class MpcEnvStep(C.Structure):
                 ("arrive_x", C.c_float), ("arrive_y", C.c_float)]
 
 
+class MpcKktOut(C.Structure):
+    _fields_ = [("residual", C.c_void_p), ("grad_norm", C.c_void_p), ("violation", C.c_void_p), ("n_active", C.c_void_p),
+                ("multipliers", C.c_void_p)]
+
+
 EXPORTS = ["mpc_create", "mpc_destroy", "mpc_last_error", "mpc_workspace_batch", "mpc_rollout_cost", "mpc_solve",
            "mpc_prepare", "mpc_predict", "mpc_predict_host", "mpc_launch_count", "mpc_fp32_peak", "mpc_timing_begin",
            "mpc_timing_end", "mpc_device_info", "mpc_set_warm_start", "mpc_set_adaptive_starts", "mpc_solve_config",
-           "mpc_env_step"]
+           "mpc_env_step", "mpc_kkt"]
 
 
 class MpcError(RuntimeError):
@@ -128,6 +133,8 @@ def load() -> C.CDLL:
     lib.mpc_solve_config.restype = C.c_int
     lib.mpc_env_step.argtypes = [C.POINTER(MpcEnvStep), vp]
     lib.mpc_env_step.restype = C.c_int
+    lib.mpc_kkt.argtypes = [vp, C.POINTER(MpcProblemBatch), C.c_int, vp, C.c_float, C.POINTER(MpcKktOut), vp]
+    lib.mpc_kkt.restype = C.c_int
     lib.mpc_device_info.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
     lib.mpc_device_info.restype = C.c_int
     _lib = lib

@@ -261,6 +261,37 @@ class BatchedPureMPC:
         self._keep = (obs, rs, w, rm)          # keep inputs alive until the stream has consumed them
         return (self.actions[:B], U) if return_controls else self.actions[:B]
 
+    def kkt_certificate(self, U: torch.Tensor, batch: Optional[Dict[str, torch.Tensor]] = None,
+                        act_tol: float = 1e-4) -> Dict[str, torch.Tensor]:
+        """FP64 first-order optimality certificate (mpc_kkt) of the controls U [B, N, 2], e.g. those of
+        `a, U = predict_batch(obs, return_controls=True)`: with g = grad_U J and the control / node bounds within act_tol of
+        their limits, residual = min over multipliers >= 0 of |g - J_act^T mu| (the oracle's kkt_residual).  batch=None
+        certifies against the problems of the last predict_batch / prepare_batch, whose B must match.  Returns device
+        tensors residual [B], grad_norm [B], violation [B], n_active [B] (int32) and multipliers [B, N, 4] (mu of a_k,
+        mu of delta_k, nu of theta_k+1, nu of v_k+1; > 0 at an upper bound, < 0 at a lower one).  Runs on the current
+        stream, no host synchronisation."""
+        if (not isinstance(U, torch.Tensor) or U.device != self.device or U.dtype != torch.float32 or not U.is_contiguous()
+                or U.dim() != 3 or tuple(U.shape[1:]) != (self.horizon, 2)):
+            raise ValueError(f"U must be a contiguous float32 [B, {self.horizon}, 2] tensor on this agent's CUDA device")
+        B = int(U.shape[0])
+        held = None
+        if batch is not None:
+            s, held, Bb = self._batch_struct(batch)
+            if Bb != B:
+                raise ValueError(f"batch has {Bb} problems, U has {B}")
+            bp = C.byref(s)
+        else:
+            bp = None
+        f32 = dict(dtype=torch.float32, device=self.device)
+        res = {"residual": torch.empty(B, **f32), "grad_norm": torch.empty(B, **f32), "violation": torch.empty(B, **f32),
+               "n_active": torch.empty(B, dtype=torch.int32, device=self.device),
+               "multipliers": torch.empty(B, self.horizon, 4, **f32)}
+        out = _capi.MpcKktOut(*(res[k].data_ptr() for k in ("residual", "grad_norm", "violation", "n_active", "multipliers")))
+        rc = self._lib.mpc_kkt(self._h, bp, B, U.data_ptr(), float(act_tol), C.byref(out), self._stream())
+        _capi.check(self._lib, self._h, rc)
+        self._keep_kkt = (U, held)
+        return res
+
     def prepare_batch(self, obs, ref_speed=None, weights=None, reset_mask=None) -> Dict[str, torch.Tensor]:
         """Parsing + collision logic only (mpc_prepare); returns the parsed-problem workspace as tensors
         (copies) for inspection / parity tests."""

@@ -18,7 +18,7 @@ LIB = os.path.join(HERE, os.environ.get("MPC_LIB_NAME", "libmpcb200.so"))      #
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",
           "--expt-relaxed-constexpr"]
-UNITS = [("mpc_solve.cu", []), ("mpc_prepare.cu", ["-fmad=false"]), ("mpc_capi.cu", []), ("mpc_env.cu", [])]
+UNITS = [("mpc_solve.cu", []), ("mpc_prepare.cu", ["-fmad=false"]), ("mpc_capi.cu", []), ("mpc_env.cu", []), ("mpc_kkt.cu", [])]
 
 
 def _nvcc() -> str:

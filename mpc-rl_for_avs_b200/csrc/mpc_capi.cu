@@ -45,6 +45,8 @@ struct MpcHandle {
   float* start_cost = nullptr;     // borrowed
   uint8_t* extended = nullptr;     // borrowed
   const float* u_init = nullptr;   // opt-in warm start (device, borrowed)
+  int last_B = -1;                 // B of the last mpc_prepare / mpc_predict(_host): the workspace's stride
+  int* kkt_block = nullptr;        // [1 + max_batch]: mpc_kkt's deferred count and list
   float* sink = nullptr;
   // host-call staging (mpc_predict_host)
   float* d_obs = nullptr; float* d_ref_speed = nullptr; float* d_weights = nullptr; uint8_t* d_reset = nullptr;
@@ -90,7 +92,7 @@ MPC_API int mpc_destroy(MpcHandle* h) {
   cudaSetDevice(h->device);
   for (auto e : h->ev_prepare) cudaEventDestroy(e);
   for (auto e : h->ev_solve) cudaEventDestroy(e);
-  cudaFree(h->ref_block); cudaFree(h->ws_block); cudaFree(h->work_counter); cudaFree(h->sink); cudaFree(h->aq_block);
+  cudaFree(h->ref_block); cudaFree(h->ws_block); cudaFree(h->work_counter); cudaFree(h->sink); cudaFree(h->aq_block); cudaFree(h->kkt_block);
   cudaFree(h->cand.cost); cudaFree(h->cand.u0); cudaFree(h->cand.status); cudaFree(h->cand.iters); cudaFree(h->cand.U);
   cudaFree(h->d_obs); cudaFree(h->d_ref_speed); cudaFree(h->d_weights); cudaFree(h->d_reset);
   cudaFree(h->d_actions); cudaFree(h->d_status); cudaFree(h->d_iters); cudaFree(h->d_cost);
@@ -248,6 +250,7 @@ MPC_API int mpc_create(const MpcConfig* cfg, int device, int max_batch, MpcHandl
     h->cand_starts = n_starts;
   }
   CKC(cudaMalloc(&h->sink, 256));
+  CKC(cudaMalloc(&h->kkt_block, (1 + B) * sizeof(int)));
   // staging for the host-buffer entry point
   CKC(cudaMalloc(&h->d_obs, B * cfg->vehicles_count * 8 * 4));
   CKC(cudaMalloc(&h->d_ref_speed, B * 4));
@@ -438,6 +441,7 @@ MPC_API int mpc_prepare(MpcHandle* h, const float* obs, const float* ref_speed, 
   int rc;
   if ((rc = timed_begin(h, h->ev_prepare, st))) return rc;
   if ((rc = prepare_range(h, obs, ref_speed, weights, reset_mask, latch, B, 0, B, col, st))) return rc;
+  h->last_B = B;
   if ((rc = timed_end(h, h->ev_prepare, st))) return rc;
   return MPC_OK;
 }
@@ -496,6 +500,7 @@ MPC_API int mpc_predict_host(MpcHandle* h, const float* obs_host, const float* r
     CK(h, cudaStreamWaitEvent(st, h->copy_done[c], 0));
     if ((rc = prepare_range(h, h->d_obs, d_rs, d_w, d_rm, &latch, B, lo, hi - lo, &col, st))) return rc;
   }
+  h->last_B = B;
   if ((rc = timed_end(h, h->ev_prepare, st))) return rc;
   MpcProblemBatch wb;
   mpc_workspace_batch(h, &wb);
@@ -521,6 +526,39 @@ MPC_API int mpc_predict_host(MpcHandle* h, const float* obs_host, const float* r
   CK(h, cudaStreamSynchronize(st));
   if (h2d_bytes) *h2d_bytes = up;
   if (d2h_bytes) *d2h_bytes = down;
+  return MPC_OK;
+}
+
+MPC_API int mpc_kkt(MpcHandle* h, const MpcProblemBatch* batch, int B, const float* U, float act_tol, const MpcKktOut* out,
+                    void* stream) {
+  if (!h) return MPC_ERR_BAD_ARG;
+  if (!U || !out || !out->residual) return fail(h, MPC_ERR_BAD_ARG, "mpc_kkt: U and out->residual are required");
+  if (!(act_tol >= 0.f)) return fail(h, MPC_ERR_BAD_ARG, "mpc_kkt: act_tol must be >= 0 and not NaN");
+  if (B < 0) return fail(h, MPC_ERR_BAD_ARG, "mpc_kkt: B < 0");
+  if (B > h->max_batch) return fail(h, MPC_ERR_TOO_LARGE, "mpc_kkt: B exceeds max_batch of mpc_create");
+  MpcProblemBatch wb;
+  if (!batch) {              // the workspace is strided by the B of the call that filled it
+    if (B != h->last_B) return fail(h, MPC_ERR_BAD_ARG, "mpc_kkt: batch == NULL needs the B of the last mpc_prepare / mpc_predict");
+    mpc_workspace_batch(h, &wb);
+    batch = &wb;
+  } else {
+    int rc = check_batch(h, batch, B);
+    if (rc) return rc;
+  }
+  if (B == 0) return MPC_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(h, cudaSetDevice(h->device));
+  CK(h, cudaMemsetAsync(h->kkt_block, 0, sizeof(int), st));
+  KktLaunch k{};
+  k.batch = *batch; k.B = B; k.N = h->scfg.N; k.M = h->scfg.M;
+  k.dt = prep_dt(h->cfg.dt);
+  k.w_distance = h->scfg.w_distance; k.w_collision = h->scfg.w_collision;
+  k.literal_no_collision = h->scfg.literal_no_collision;
+  k.ref = h->tables.ref; k.U = U; k.act_tol = (double)act_tol; k.out = *out;
+  k.n_deferred = h->kkt_block; k.deferred = h->kkt_block + 1;
+  k.grid_deferred = h->sm_count * 2;
+  CK(h, launch_kkt(k, st));
+  h->launches += 2;
   return MPC_OK;
 }
 

@@ -106,4 +106,21 @@ cudaError_t launch_solve_tmem(const SolveLaunch& s, cudaStream_t stream);
 cudaError_t launch_select(const SolveLaunch& s, cudaStream_t stream);
 cudaError_t launch_select_adaptive(const SolveLaunch& s, cudaStream_t stream);
 
+// defined in mpc_kkt.cu: the optimality certificate of controls U (mpc_kkt)
+struct KktLaunch {
+  MpcProblemBatch batch;
+  int B, N, M;
+  double dt;              // the double 1 / policy_frequency
+  double w_distance, w_collision;
+  int literal_no_collision;
+  const double* ref;      // RefTables::ref
+  const float* U;         // [B][N][2]
+  double act_tol;
+  MpcKktOut out;
+  int* n_deferred;        // device, zeroed before launch: problems handed to k_kkt_deferred
+  int* deferred;          // [B] their indices
+  int grid_deferred;
+};
+cudaError_t launch_kkt(const KktLaunch& k, cudaStream_t stream);
+
 }  // namespace mpcb
