@@ -902,6 +902,21 @@ MPC_PRAGMA_UNROLL_OBS
   *d2_out = d2;
 }
 
+// ---- control of one stage under the affine policy ----------------------------------------------
+// (ac, dc) = u_nom + alpha k + K dz clamped to the box of the node at (th, v); dz = (ex, ey, eth, ev, dap, ddp) is the
+// deviation from the nominal state and the previous stage's control change.  Returns the steering terms of dc.
+template <typename T>
+MPC_HD Steer<T> policy_control(const T (&Kr)[12], T f0, T f1, T alpha, T ex, T ey, T eth, T ev, T dap, T ddp, bool open_loop,
+                               T th, T v, T dt, T ua, T ud, T& ac, T& dc) {
+  T da = alpha * f0 + Kr[0] * ex + Kr[1] * ey + Kr[2] * eth + Kr[3] * ev + Kr[4] * dap + Kr[5] * ddp;
+  T dd = alpha * f1 + Kr[6] * ex + Kr[7] * ey + Kr[8] * eth + Kr[9] * ev + Kr[10] * dap + Kr[11] * ddp;
+  if (open_loop) { da = T(0); dd = T(0); }
+  const Box<T> bx = control_box(th, v, dt);
+  ac = clamp_(ua + da, bx.lo_a, bx.hi_a);
+  dc = ud + dd;
+  return clamp_steer(bx, dc, false);
+}
+
 // ---- closed-loop forward pass -----------------------------------------------------------------
 // Rolls the dynamics forward under the affine policy u = u_nom + alpha k + K dz, clamped to the
 // node's control box, for NA step lengths AT ONCE (independent dependency chains: the kernel is
@@ -930,14 +945,9 @@ MPC_HD void forward_pass(const SolverConfig& cfg, const ProblemScalars<T>& p, co
     sl.load_gains(k, f0, f1, Kr);
 #pragma unroll
     for (int a = 0; a < NA; ++a) {
-      const T ex = x[a] - xn, ey = y[a] - yn, eth = th[a] - thn, ev = v[a] - vn;
-      T da = alpha[a] * f0 + Kr[0] * ex + Kr[1] * ey + Kr[2] * eth + Kr[3] * ev + Kr[4] * dap[a] + Kr[5] * ddp[a];
-      T dd = alpha[a] * f1 + Kr[6] * ex + Kr[7] * ey + Kr[8] * eth + Kr[9] * ev + Kr[10] * dap[a] + Kr[11] * ddp[a];
-      if (open_loop) { da = T(0); dd = T(0); }
-      const Box<T> bx = control_box(th[a], v[a], dt);
-      const T ac = clamp_(ua + da, bx.lo_a, bx.hi_a);
-      T dc = ud + dd;
-      const Steer<T> st = clamp_steer(bx, dc, false);
+      T ac, dc;
+      const Steer<T> st = policy_control(Kr, f0, f1, alpha[a], x[a] - xn, y[a] - yn, th[a] - thn, v[a] - vn, dap[a], ddp[a],
+                                         open_loop, th[a], v[a], dt, ua, ud, ac, dc);
       dap[a] = ac - ua; ddp[a] = dc - ud;
       maxdu[a] = max_(maxdu[a], max_(abs_(dap[a]), abs_(ddp[a])));
       if (with_cost) J[a] += stage_cost(cfg, p, ref, sl, k, x[a], y[a], th[a], v[a], ac, dc, ap[a], dp[a], (T*)nullptr);
@@ -950,6 +960,17 @@ MPC_HD void forward_pass(const SolverConfig& cfg, const ProblemScalars<T>& p, co
     }
   }
   if (NA == 1 && commit) { sl.X(N, 0) = x[0]; sl.X(N, 1) = y[0]; sl.X(N, 2) = th[0]; sl.X(N, 3) = v[0]; }
+}
+
+// The control that the commit sweep forward_pass<T, 1>(alpha, commit) would store in U(0), without the sweep: the same
+// operations on the same operands (the state deviations x - x of stage 0 included), so the same bits, inf / NaN gains too.
+template <typename T, typename SL>
+MPC_HD void first_control(const SolverConfig& cfg, const SL& sl, T alpha, T& ac, T& dc) {
+  const T x = sl.X(0, 0), y = sl.X(0, 1), th = sl.X(0, 2), v = sl.X(0, 3);
+  T f0, f1, Kr[12];
+  sl.load_gains(0, f0, f1, Kr);
+  policy_control(Kr, f0, f1, alpha, x - x, y - y, th - th, v - v, T(0), T(0), false, th, v, T(cfg.dt), sl.U(0, 0), sl.U(0, 1),
+                 ac, dc);
 }
 
 // status bits returned per problem

@@ -13,7 +13,8 @@
 //     that finishes pulls the next problem index from a global counter (after a static first wave)
 //     instead of idling until its warp's slowest problem ends.
 //   * one trip of the loop = backward sweep, ONE line-search sweep of two candidates (alpha, alpha/4),
-//     commit sweep; a rejected step raises the Levenberg damping for the next trip.
+//     commit sweep (k_solve_tmem: the lead sweep of the next trip); a rejected step raises the Levenberg damping
+//     for the next trip.
 //   * the tail of a launch (k_solve_tmem, 192/256 threads): the surviving problems are packed into the
 //     lowest warps, and the freed lanes run the trips the sequential algorithm would run after 1, 2, ...
 //     rejections side by side (see the comments at kCompact / kSpec).
@@ -100,14 +101,15 @@ __device__ __forceinline__ void begin_item(const SolverConfig& cfg, const MpcPro
     }
   }
 }
-// result of a finished item: straight to the caller's arrays (one start) or to the candidate arrays (portfolio)
+// result of a finished item: straight to the caller's arrays (one start) or to the candidate arrays (portfolio).
+// (u0a, u0d) is the first control; the full controls (out.U) are read from the slots.
 template <typename SL>
 __device__ __forceinline__ void finish_item(const SolverConfig& cfg, const MpcSolveOut& out, const SolveCand& cand, int n_starts, int idx,
-                                            const SL& sl, SolveState<float>& s) {
+                                            const SL& sl, SolveState<float>& s, float u0a, float u0d) {
   if (!(s.J == s.J)) s.status |= kStatusNaN;
   if (n_starts == 1) {
-    out.actions[2 * (size_t)idx] = sl.U(0, 0);
-    out.actions[2 * (size_t)idx + 1] = sl.U(0, 1);
+    out.actions[2 * (size_t)idx] = u0a;
+    out.actions[2 * (size_t)idx + 1] = u0d;
     if (out.status) out.status[idx] = s.status;
     if (out.iters) out.iters[idx] = s.iter;
     if (out.cost) out.cost[idx] = s.J;
@@ -118,8 +120,8 @@ __device__ __forceinline__ void finish_item(const SolverConfig& cfg, const MpcSo
         out.U[((size_t)idx * cfg.N + k) * 2 + 1] = sl.U(k, 1);
       }
   } else {
-    cand.u0[2 * (size_t)idx] = sl.U(0, 0);
-    cand.u0[2 * (size_t)idx + 1] = sl.U(0, 1);
+    cand.u0[2 * (size_t)idx] = u0a;
+    cand.u0[2 * (size_t)idx + 1] = u0d;
     cand.status[idx] = s.status;
     cand.iters[idx] = s.iter;
     cand.cost[idx] = s.J;
@@ -250,7 +252,7 @@ k_solve(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut o
       } else {
         after_line_search(cfg, s, acc, alpha, Jn, md, alpha * d1 + alpha * alpha * d2);
         if (s.done) {
-          finish_item(cfg, out, cand, n_starts, idx, sl, s);
+          finish_item(cfg, out, cand, n_starts, idx, sl, s, sl.U(0, 0), sl.U(0, 1));
           if constexpr (kAdaptive) if (idx < B * n_starts) publish_base(aq, cand, B, n_starts, idx);
           active = false;
           need_fetch = true;
@@ -261,7 +263,13 @@ k_solve(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut o
 }
 
 // ---- variant with the gains in tensor memory -----------------------------------------------------
-// Same trip structure; differences forced by the warp-collective tcgen05.ld/st:
+// The trip is rotated so that a lane can start a new item in the trip that fetches it:
+//   lead sweep (commit of the previous trip's accepted step, or the open-loop first rollout of a fresh item)
+//   -> block barrier / tail compaction -> backward sweep -> line-search sweep -> bookkeeping -> finish and fetch.
+// An item that ends on an accepted step skips that step's commit: its first control is stage 0 of the commit
+// (first_control), its objective the line search's.  Only when the full controls are returned (out.U) does it commit in
+// the next lead sweep and finish after it.
+// Differences forced by the warp-collective tcgen05.ld/st:
 //   * every sweep is executed by all 32 lanes whenever ANY lane needs it.  Lanes without work compute on
 //     whatever their slots hold (finite loops only, results discarded); their TMEM stores land in their own
 //     cells.  Under SIMT those lanes were waiting anyway.
@@ -332,6 +340,9 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
   int idx = -1;
   bool active = false, fresh = false, need_fetch = true, first_wave = true;
   bool pending = false;                                     // kAdaptive: holds a ticket whose slot is not written yet
+  bool commit = false;                                      // this lane's step was accepted last trip: the lead sweep commits it
+  float alpha_c = 1.f;                                      // with this step length (the gains are still in this lane's TMEM cells)
+  const bool full_controls = out.U != nullptr;              // out.U and cand.U: the item's controls are returned, not only U(0)
 
   for (;;) {
     if (need_fetch) {
@@ -368,6 +379,18 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
         }
       }
     }
+    // ---- lead sweep.  Before the barrier: no commit is pending when compaction moves register state between lanes.
+    const bool lead = fresh || commit;
+    float Jc = 0.f, mdc = 0.f;
+    if (__any_sync(full, lead)) {                           // all 32 lanes sweep; only `lead` lanes write
+      forward_pass<float, 1, SL>(cfg, p, ref, sl, &alpha_c, lead, fresh, fresh, &Jc, &mdc);
+      __syncwarp();
+    }
+    if (fresh) {
+      solve_init_finish(s, Jc);
+      fresh = false;
+    }
+    commit = false;
     __syncwarp();
     if (kCompact) {
       // ---- one block barrier per trip: count the running problems; once the queue is drained and they fit
@@ -423,7 +446,7 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
           q[16] = __float_as_uint(s.md_last);
           q[17] = __float_as_uint(s.J_mark); q[18] = (uint32_t)s.iter; q[19] = (uint32_t)s.status;
           q[20] = (uint32_t)s.trials; q[21] = (uint32_t)s.fails;
-          q[22] = (uint32_t)idx; q[23] = fresh ? 1u : 0u;
+          q[22] = (uint32_t)idx; q[23] = s.done ? 1u : 0u;
           q[24] = (uint32_t)(sl.base - slot0);               // the shared-memory column that holds U, X, obstacles
         }
         __syncthreads();
@@ -431,7 +454,6 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
         spec_k = k_new;
         spec_j = (int)threadIdx.x % k_new;
         active = group < n_active;
-        fresh = false;
         if (active) {
           const uint32_t* q = scratch + group * kCompactWords;
           p.x0 = __hiloint2double((int)q[1], (int)q[0]); p.y0 = __hiloint2double((int)q[3], (int)q[2]);
@@ -441,8 +463,8 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
           p.vr_n = (int)q[13];
           s.J = __uint_as_float(q[14]); s.mu = __uint_as_float(q[15]); s.md_last = __uint_as_float(q[16]);
           s.J_mark = __uint_as_float(q[17]); s.iter = (int)q[18]; s.status = (int)q[19];
-          s.trials = (int)q[20]; s.fails = (int)q[21]; s.done = false;
-          idx = (int)q[22]; fresh = q[23] != 0u;
+          s.trials = (int)q[20]; s.fails = (int)q[21]; s.done = q[23] != 0u;
+          idx = (int)q[22];
           sl.base = slot0 + q[24];
         } else {
           spec_j = 0;                                        // idle lanes must not look like followers of a group
@@ -456,7 +478,7 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
     }
     float d1 = 0.f, d2 = 0.f, alpha = 1.f, Jn = 0.f, md = 0.f;
     bool ok = false;
-    const bool run = active && !fresh;
+    const bool run = active && !s.done;                     // a done item here was committed by the lead sweep: it only finishes
     const bool any_run = __any_sync(full, run);
     const int trials0 = s.trials;
     if (any_run) {                                          // all 32 lanes sweep; only `run` lanes keep the result
@@ -467,16 +489,18 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
       ok = line_search_pass(cfg, p, ref, sl, s, d1, d2, alpha, Jn, md) && run;
       __syncwarp();
     }
-    // ---- bookkeeping of the solver state (before the commit sweep: it only needs the line-search results)
-    bool commit_me = false;
+    // ---- bookkeeping of the solver state
+    bool acc = false;                                       // the problem's step was accepted (in a group: some lane's)
+    bool commit_me = false;                                 // ... and this lane holds its gains
+    int src = 0;                                            // group lane whose gains made the accepted step
     if (!kSpec || spec_k == 1) {
-      if (run) { after_line_search(cfg, s, ok, alpha, Jn, md, alpha * d1 + alpha * alpha * d2); commit_me = ok; }
+      if (run) { after_line_search(cfg, s, ok, alpha, Jn, md, alpha * d1 + alpha * alpha * d2); acc = commit_me = ok; }
     } else {
       const unsigned okmask = __ballot_sync(full, ok);
       const int gbase = (threadIdx.x & 31) & ~(spec_k - 1);
       const unsigned gm = (okmask >> gbase) & ((1u << spec_k) - 1u);
       const int w = gm ? (__ffs((int)gm) - 1) : spec_k;     // first speculative lane whose step was accepted
-      const int src = gbase + (w < spec_k ? w : 0);
+      src = gbase + (w < spec_k ? w : 0);
       const float a_w = __shfl_sync(full, alpha, src), J_w = __shfl_sync(full, Jn, src), md_w = __shfl_sync(full, md, src);
       const float ex_w = __shfl_sync(full, alpha * d1 + alpha * alpha * d2, src);
       if (run) {
@@ -487,29 +511,31 @@ k_solve_tmem(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolve
           after_line_search(cfg, s, false, 1.f, 0.f, 0.f, 0.f);
         }
         s.trials = trials0 + MPC_LS_NA * t;
+        acc = reached;
         commit_me = reached && spec_j == w;
       }
     }
-    const bool do_commit = active && (fresh ? spec_j == 0 : commit_me);
-    float Jc = 0.f, mdc = 0.f;
-    if (__any_sync(full, do_commit)) {
-      forward_pass<float, 1, SL>(cfg, p, ref, sl, &alpha, do_commit, fresh, fresh, &Jc, &mdc);
-      __syncwarp();
+    // ---- finish and fetch.  An item that ends on a rejected step returns U(0) as it is; one that ends on an accepted
+    // step returns stage 0 of that step's commit, unless its full controls are wanted: then it is `deferred`.
+    const bool ends = run && s.done;
+    const bool deferred = ends && acc && full_controls;
+    const bool u0_policy = ends && acc && !full_controls;
+    commit = commit_me && (!ends || deferred);
+    alpha_c = alpha;
+    float u0a = 0.f, u0d = 0.f;
+    if (__any_sync(full, u0_policy)) {                      // tcgen05.ld: all 32 lanes
+      first_control(cfg, sl, alpha, u0a, u0d);
+      if (kSpec && spec_k > 1) { u0a = __shfl_sync(full, u0a, src); u0d = __shfl_sync(full, u0d, src); }
     }
-    if (kSpec && spec_k > 1) Jc = __shfl_sync(full, Jc, (threadIdx.x & 31) & ~(spec_k - 1));   // the group leader did the first rollout
-    if (active) {
-      if (fresh) {
-        solve_init_finish(s, Jc);
-        fresh = false;
-      } else if (s.done) {
-        if (spec_j == 0) {
-          finish_item(cfg, out, cand, n_starts, idx, sl, s);
-          if constexpr (kAdaptive) if (idx < B * n_starts) publish_base(aq, cand, B, n_starts, idx);
-        }
-        active = false;
-        spec_j = 0;
-        need_fetch = !drained;                               // nothing left to fetch once a lane of the block saw the queue empty
+    if (active && s.done && !deferred) {
+      if (spec_j == 0) {
+        if (!u0_policy) { u0a = sl.U(0, 0); u0d = sl.U(0, 1); }
+        finish_item(cfg, out, cand, n_starts, idx, sl, s, u0a, u0d);
+        if constexpr (kAdaptive) if (idx < B * n_starts) publish_base(aq, cand, B, n_starts, idx);
       }
+      active = false;
+      spec_j = 0;
+      need_fetch = !drained;                                 // nothing left to fetch once a lane of the block saw the queue empty
     }
   }
   asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
