@@ -109,6 +109,29 @@ MPC_HD float sqrt_(float x) { return sqrtf(x); }
 MPC_HD double sqrt_(double x) { return sqrt(x); }
 MPC_HD float abs_(float x) { return fabsf(x); }
 MPC_HD double abs_(double x) { return fabs(x); }
+// ---- two lanes of one expression: the line search's two candidates (forward_pass<T, 2>) -------------------
+// On the device a float pair is evaluated by one packed FP32 instruction per operation (sm_100 FADD2 / FMUL2 / FFMA2,
+// round-to-nearest, no flush to zero): per lane it is the same IEEE operation as the scalar code.  The packed forms are
+// never contracted by the compiler, so an expression is written with fma2 exactly where the scalar code's multiply-add
+// was fused, and with mul2 + add2 where it was not.  The host (and T = double) evaluates two plain scalar expressions,
+// as it compiles the scalar code: no std::fma.
+template <typename T> struct Pair { T a, b; };
+template <typename T> MPC_HD Pair<T> splat(T x) { return {x, x}; }
+template <typename T> MPC_HD Pair<T> add2(Pair<T> x, Pair<T> y) { return {x.a + y.a, x.b + y.b}; }
+template <typename T> MPC_HD Pair<T> mul2(Pair<T> x, Pair<T> y) { return {x.a * y.a, x.b * y.b}; }
+template <typename T> MPC_HD Pair<T> fma2(Pair<T> x, Pair<T> y, Pair<T> z) { return {x.a * y.a + z.a, x.b * y.b + z.b}; }
+#if defined(__CUDA_ARCH__)
+__device__ __forceinline__ float2 f2_(Pair<float> x) { return make_float2(x.a, x.b); }
+__device__ __forceinline__ Pair<float> add2(Pair<float> x, Pair<float> y) { const float2 r = __fadd2_rn(f2_(x), f2_(y)); return {r.x, r.y}; }
+__device__ __forceinline__ Pair<float> mul2(Pair<float> x, Pair<float> y) { const float2 r = __fmul2_rn(f2_(x), f2_(y)); return {r.x, r.y}; }
+__device__ __forceinline__ Pair<float> fma2(Pair<float> x, Pair<float> y, Pair<float> z) {
+  const float2 r = __ffma2_rn(f2_(x), f2_(y), f2_(z));
+  return {r.x, r.y};
+}
+#endif
+// x - y as x + (-y): the same IEEE result
+template <typename T> MPC_HD Pair<T> sub2(Pair<T> x, Pair<T> y) { return add2(x, Pair<T>{-y.a, -y.b}); }
+
 template <typename T> MPC_HD T min_(T a, T b) { return a < b ? a : b; }
 template <typename T> MPC_HD T max_(T a, T b) { return a > b ? a : b; }
 template <typename T> MPC_HD T clamp_(T x, T lo, T hi) { return min_(max_(x, lo), hi); }
@@ -394,6 +417,51 @@ MPC_PRAGMA_UNROLL_OBS
   if (comp) { comp[0] += st; comp[1] += ct; comp[3] += df; comp[4] += dist; comp[5] += col; }
   if (cfg.literal_no_collision) return p.w_control * ct + p.w_diff * df;
   return T(10) * st + p.w_control * ct + p.w_diff * df + T(cfg.w_distance) * dist + T(cfg.w_collision) * col;
+}
+
+// stage_cost of the line search's two candidates at once (no components): the same operations on each lane, with the
+// multiply-adds fused exactly where the device build of stage_cost fuses them inside forward_pass<T, 2> (read from its
+// SASS of every solve kernel; e.g. the input-difference sum is fma(ed, ed, ea^2) there but fma(ea, ea, ed^2) in the
+// single-candidate sweep).  The scalar code fuses `para` differently per slot type: fma(dy, sh, dx ch) where the path
+// positions are staged in the problem's column (SlotsTmem, k_solve_tmem), fma(dx, ch, dy sh) where they are read from
+// the block's table (Slots, k_solve).  The shared operands (reference point, reference speed, obstacle tracks) are
+// broadcast once per stage and obstacle; rsqrt_ and the selects stay per lane.
+template <typename T, typename SL>
+MPC_HD Pair<T> stage_cost2(const SolverConfig& cfg, const ProblemScalars<T>& p, const RefTab<T>& ref, const SL& sl, int k,
+                           Pair<T> x, Pair<T> y, Pair<T> th, Pair<T> v, Pair<T> a, Pair<T> d, Pair<T> ap, Pair<T> dp) {
+  const RefPoint<T> r = ref_point(ref, p, sl, k);
+  const Pair<T> sh = splat(r.sh), ch = splat(r.ch);
+  const Pair<T> dx = add2(x, splat(-r.x)), dy = add2(y, splat(-r.y));
+  const Pair<T> perp = fma2(dx, sh, mul2(dy, splat(-r.ch)));     // dx sh - dy ch
+  const Pair<T> para = SL::kRefStaged ? fma2(dy, sh, mul2(dx, ch)) : fma2(dx, ch, mul2(dy, sh));   // dx ch + dy sh
+  const Pair<T> dv = add2(v, splat(-ref_speed_at(p, k)));
+  const Pair<T> dth = add2(th, splat(-r.h));
+  Pair<T> st = fma2(perp, mul2(perp, splat(T(4))), mul2(para, add2(para, para)));
+  st = fma2(dv, mul2(splat(p.w_speed), dv), st);
+  st = fma2(dth, mul2(dth, splat(T(0.5))), st);
+  const Pair<T> ct = mul2(fma2(a, a, mul2(d, d)), splat(T(0.01)));
+  Pair<T> df = splat(T(0));
+  if (k > 0) { const Pair<T> ea = sub2(a, ap), ed = sub2(d, dp); df = mul2(fma2(ed, ed, mul2(ea, ea)), splat(T(0.01))); }
+  Pair<T> dist = splat(T(0));
+  if (cfg.w_distance != 0.f) {
+    const Pair<T> nkf = splat(-T(k));
+    const Pair<T> tiny = splat(T(1e-30)), one = splat(T(1)), neps = splat(-T(2e-6));
+MPC_PRAGMA_UNROLL_OBS
+    for (int m = 0; m < p.n_obs; ++m) {
+      const Pair<T> ex = fma2(nkf, splat(sl.O(m, 2)), add2(x, splat(-sl.O(m, 0))));
+      const Pair<T> ey = fma2(nkf, splat(sl.O(m, 3)), add2(y, splat(-sl.O(m, 1))));
+      const Pair<T> d2 = fma2(ex, ex, fma2(ey, ey, tiny));
+      const Pair<T> idd = {rsqrt_(d2.a), rsqrt_(d2.b)};
+      const Pair<T> c = {d2.a < T(1) ? T(1000) : T(100), d2.b < T(1) ? T(1000) : T(100)};
+      dist = fma2(mul2(c, mul2(idd, idd)), fma2(idd, neps, one), dist);
+    }
+  }
+  const Pair<T> col = p.is_collide ? mul2(mul2(v, splat(T(3000))), v) : splat(T(0));
+  if (cfg.literal_no_collision) return fma2(splat(p.w_control), ct, mul2(splat(p.w_diff), df));
+  Pair<T> J = fma2(splat(p.w_control), ct, mul2(st, splat(T(10))));
+  J = fma2(splat(p.w_diff), df, J);
+  J = fma2(dist, splat(T(cfg.w_distance)), J);
+  return fma2(col, splat(T(cfg.w_collision)), J);
 }
 
 // ---- state bounds as state-dependent control boxes ------------------------------------------
@@ -943,20 +1011,45 @@ MPC_HD void forward_pass(const SolverConfig& cfg, const ProblemScalars<T>& p, co
     const T ua = sl.U(k, 0), ud = sl.U(k, 1);
     T f0, f1, Kr[12];
     sl.load_gains(k, f0, f1, Kr);
+    if constexpr (NA == 2) {
+      // both candidates' controls first, then their stage costs as one packed evaluation, then their Euler steps
+      T ac[2], dc[2];
+      Steer<T> st[2];
 #pragma unroll
-    for (int a = 0; a < NA; ++a) {
-      T ac, dc;
-      const Steer<T> st = policy_control(Kr, f0, f1, alpha[a], x[a] - xn, y[a] - yn, th[a] - thn, v[a] - vn, dap[a], ddp[a],
-                                         open_loop, th[a], v[a], dt, ua, ud, ac, dc);
-      dap[a] = ac - ua; ddp[a] = dc - ud;
-      maxdu[a] = max_(maxdu[a], max_(abs_(dap[a]), abs_(ddp[a])));
-      if (with_cost) J[a] += stage_cost(cfg, p, ref, sl, k, x[a], y[a], th[a], v[a], ac, dc, ap[a], dp[a], (T*)nullptr);
-      if (NA == 1 && commit) {
-        sl.X(k, 0) = x[a]; sl.X(k, 1) = y[a]; sl.X(k, 2) = th[a]; sl.X(k, 3) = v[a];
-        sl.U(k, 0) = ac; sl.U(k, 1) = dc;
+      for (int a = 0; a < 2; ++a) {
+        st[a] = policy_control(Kr, f0, f1, alpha[a], x[a] - xn, y[a] - yn, th[a] - thn, v[a] - vn, dap[a], ddp[a],
+                               open_loop, th[a], v[a], dt, ua, ud, ac[a], dc[a]);
+        dap[a] = ac[a] - ua; ddp[a] = dc[a] - ud;
+        maxdu[a] = max_(maxdu[a], max_(abs_(dap[a]), abs_(ddp[a])));
       }
-      euler_step(x[a], y[a], th[a], v[a], ac, st, dt);
-      ap[a] = ac; dp[a] = dc;
+      if (with_cost) {
+        const Pair<T> c = stage_cost2(cfg, p, ref, sl, k, Pair<T>{x[0], x[1]}, Pair<T>{y[0], y[1]}, Pair<T>{th[0], th[1]},
+                                      Pair<T>{v[0], v[1]}, Pair<T>{ac[0], ac[1]}, Pair<T>{dc[0], dc[1]}, Pair<T>{ap[0], ap[1]},
+                                      Pair<T>{dp[0], dp[1]});
+        const Pair<T> Js = add2(Pair<T>{J[0], J[1]}, c);
+        J[0] = Js.a; J[1] = Js.b;
+      }
+#pragma unroll
+      for (int a = 0; a < 2; ++a) {
+        euler_step(x[a], y[a], th[a], v[a], ac[a], st[a], dt);
+        ap[a] = ac[a]; dp[a] = dc[a];
+      }
+    } else {
+#pragma unroll
+      for (int a = 0; a < NA; ++a) {
+        T ac, dc;
+        const Steer<T> st = policy_control(Kr, f0, f1, alpha[a], x[a] - xn, y[a] - yn, th[a] - thn, v[a] - vn, dap[a], ddp[a],
+                                           open_loop, th[a], v[a], dt, ua, ud, ac, dc);
+        dap[a] = ac - ua; ddp[a] = dc - ud;
+        maxdu[a] = max_(maxdu[a], max_(abs_(dap[a]), abs_(ddp[a])));
+        if (with_cost) J[a] += stage_cost(cfg, p, ref, sl, k, x[a], y[a], th[a], v[a], ac, dc, ap[a], dp[a], (T*)nullptr);
+        if (NA == 1 && commit) {
+          sl.X(k, 0) = x[a]; sl.X(k, 1) = y[a]; sl.X(k, 2) = th[a]; sl.X(k, 3) = v[a];
+          sl.U(k, 0) = ac; sl.U(k, 1) = dc;
+        }
+        euler_step(x[a], y[a], th[a], v[a], ac, st, dt);
+        ap[a] = ac; dp[a] = dc;
+      }
     }
   }
   if (NA == 1 && commit) { sl.X(N, 0) = x[0]; sl.X(N, 1) = y[0]; sl.X(N, 2) = th[0]; sl.X(N, 3) = v[0]; }

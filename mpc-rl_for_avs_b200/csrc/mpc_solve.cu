@@ -273,8 +273,9 @@ k_solve(const SolverConfig cfg, const MpcProblemBatch batch, const MpcSolveOut o
 //   * every sweep is executed by all 32 lanes whenever ANY lane needs it.  Lanes without work compute on
 //     whatever their slots hold (finite loops only, results discarded); their TMEM stores land in their own
 //     cells.  Under SIMT those lanes were waiting anyway.
-//   * shared memory per problem is 156 words -> up to 352 problems fit an SM (192 with gains in shared memory);
-//     256 are used, which leaves room for the scratch of the tail compaction.
+//   * shared memory per problem is 196 words at H=20, M=8 (U, X, obstacle tracks and the problem's path column) -> up
+//     to 288 problems fit an SM (192 with gains in shared memory); 256 are used, which leaves room for the scratch of
+//     the tail compaction.
 constexpr int kTmemColsPerStage = 8;
 // Tail compaction (k_solve_tmem, blocks of <= 256 threads): scratch for moving up to kCompactMax problems'
 // register state between lanes, plus one counter per warp.
