@@ -217,6 +217,33 @@ typedef struct MpcKktOut {
 MPC_API int mpc_kkt(MpcHandle* h, const MpcProblemBatch* batch, int B, const float* U, float act_tol, const MpcKktOut* out,
                     void* stream);
 
+/* Sensitivity of the first control to the problem-level parameters the RL policy sets, for controls U [B][N][2] at a
+ * local optimum (e.g. MpcSolveOut.U of a solve), in FP64 per problem: jac = dU_0 / dp (2 x 4, rows a_0, delta_0) with
+ * p = (vr_b, w_speed, w_control, w_diff) of MpcProblemBatch; vr_b is the reference speed of the stages k >= vr_n (all
+ * stages under an RL ref_speed override).  The implicit-function theorem on the KKT system with the active set of mpc_kkt
+ * held fixed (control bounds, theta / v bounds of nodes 1..N within act_tol) and the exact Hessian of the Lagrangian,
+ * solved by one O(N) constrained Riccati sweep per problem.
+ * flags: 0 = the derivative of the local optimum; otherwise MPC_SENS_* bits, jac NaN unless only WEAKLY_ACTIVE is set:
+ *   NOT_STATIONARY  stationarity residual over the free coordinates > stat_tol (1 + |J|), or a multiplier < -1e-6 (1 + |J|)
+ *   WEAKLY_ACTIVE   an active bound's multiplier is within 1e-6 (1 + |J|) of 0: jac is the one-sided derivative of the
+ *                   piece that keeps the bound active
+ *   DEGENERATE      the active constraint gradients are linearly dependent (LICQ fails)
+ *   NOT_SOSC        the Hessian reduced to the null space of the active rows is not positive definite
+ *   NONFINITE       the controls, the rollout or the gradient are not finite
+ * batch == NULL uses the handle's workspace, whose B it must repeat (as mpc_kkt).  act_tol and stat_tol must be >= 0 and
+ * not NaN.  No allocation and no host synchronisation (capturable in a CUDA graph). */
+#define MPC_SENS_NOT_STATIONARY 1
+#define MPC_SENS_WEAKLY_ACTIVE 2
+#define MPC_SENS_DEGENERATE 4
+#define MPC_SENS_NOT_SOSC 8
+#define MPC_SENS_NONFINITE 16
+typedef struct MpcSensOut {
+  float* jac;                 /* [B][2][4]  d(a_0, delta_0) / d(vr_b, w_speed, w_control, w_diff) */
+  int32_t* flags;             /* [B]        MPC_SENS_* bits */
+} MpcSensOut;
+MPC_API int mpc_sensitivity(MpcHandle* h, const MpcProblemBatch* batch, int B, const float* U, float act_tol,
+                            float stat_tol, const MpcSensOut* out, void* stream);
+
 /* Measurement helpers */
 /* number of this library's kernel launches since mpc_create (bench.py's gpu_launches) */
 MPC_API int64_t mpc_launch_count(const MpcHandle* h);

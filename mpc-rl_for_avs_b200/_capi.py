@@ -72,10 +72,17 @@ class MpcKktOut(C.Structure):
                 ("multipliers", C.c_void_p)]
 
 
+class MpcSensOut(C.Structure):
+    _fields_ = [("jac", C.c_void_p), ("flags", C.c_void_p)]
+
+
+SENS_NOT_STATIONARY, SENS_WEAKLY_ACTIVE, SENS_DEGENERATE, SENS_NOT_SOSC, SENS_NONFINITE = 1, 2, 4, 8, 16
+
+
 EXPORTS = ["mpc_create", "mpc_destroy", "mpc_last_error", "mpc_workspace_batch", "mpc_rollout_cost", "mpc_solve",
            "mpc_prepare", "mpc_predict", "mpc_predict_host", "mpc_launch_count", "mpc_fp32_peak", "mpc_timing_begin",
            "mpc_timing_end", "mpc_device_info", "mpc_set_warm_start", "mpc_set_adaptive_starts", "mpc_solve_config",
-           "mpc_env_step", "mpc_kkt"]
+           "mpc_env_step", "mpc_kkt", "mpc_sensitivity"]
 
 
 class MpcError(RuntimeError):
@@ -135,6 +142,8 @@ def load() -> C.CDLL:
     lib.mpc_env_step.restype = C.c_int
     lib.mpc_kkt.argtypes = [vp, C.POINTER(MpcProblemBatch), C.c_int, vp, C.c_float, C.POINTER(MpcKktOut), vp]
     lib.mpc_kkt.restype = C.c_int
+    lib.mpc_sensitivity.argtypes = [vp, C.POINTER(MpcProblemBatch), C.c_int, vp, C.c_float, C.c_float, C.POINTER(MpcSensOut), vp]
+    lib.mpc_sensitivity.restype = C.c_int
     lib.mpc_device_info.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
     lib.mpc_device_info.restype = C.c_int
     _lib = lib

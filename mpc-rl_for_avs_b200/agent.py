@@ -118,6 +118,7 @@ class BatchedPureMPC:
         self.max_starts = 0
         self.start_cost = None
         self.extended = None
+        self.sens_flags = torch.zeros(B, dtype=torch.int32, device=dev)
 
     # ------------------------------------------------------------------ lifecycle
     def close(self) -> None:
@@ -291,6 +292,46 @@ class BatchedPureMPC:
         _capi.check(self._lib, self._h, rc)
         self._keep_kkt = (U, held)
         return res
+
+    def sensitivity(self, U: torch.Tensor, batch: Optional[Dict[str, torch.Tensor]] = None, act_tol: float = 1e-4,
+                    stat_tol: float = 1e-3) -> Dict[str, torch.Tensor]:
+        """FP64 sensitivity (mpc_sensitivity) of the first control of the local optimum U [B, N, 2] to the problem
+        parameters p = (vr_b, w_speed, w_control, w_diff) of the batch: jac [B, 2, 4] = d(a_0, delta_0) / dp, with the
+        active set (bounds within act_tol, as kkt_certificate) held fixed.  flags [B] (int32, _capi.SENS_* bits): 0 = the
+        derivative of the local optimum; WEAKLY_ACTIVE alone = the one-sided derivative of the piece that keeps a weakly
+        active bound active; any other bit = no derivative (jac NaN).  batch=None uses the problems of the last
+        predict_batch / prepare_batch, whose B must match.  Runs on the current stream, no host synchronisation."""
+        if (not isinstance(U, torch.Tensor) or U.device != self.device or U.dtype != torch.float32 or not U.is_contiguous()
+                or U.dim() != 3 or tuple(U.shape[1:]) != (self.horizon, 2)):
+            raise ValueError(f"U must be a contiguous float32 [B, {self.horizon}, 2] tensor on this agent's CUDA device")
+        B = int(U.shape[0])
+        held = None
+        if batch is not None:
+            s, held, Bb = self._batch_struct(batch)
+            if Bb != B:
+                raise ValueError(f"batch has {Bb} problems, U has {B}")
+            bp = C.byref(s)
+        else:
+            bp = None
+        res = {"jac": torch.empty(B, 2, 4, dtype=torch.float32, device=self.device),
+               "flags": torch.empty(B, dtype=torch.int32, device=self.device)}
+        out = _capi.MpcSensOut(res["jac"].data_ptr(), res["flags"].data_ptr())
+        rc = self._lib.mpc_sensitivity(self._h, bp, B, U.data_ptr(), float(act_tol), float(stat_tol), C.byref(out),
+                                       self._stream())
+        _capi.check(self._lib, self._h, rc)
+        self._keep_sens = (U, held)
+        return res
+
+    def predict_batch_autograd(self, obs: torch.Tensor, ref_speed: Optional[torch.Tensor] = None,
+                               weights: Optional[torch.Tensor] = None, reset_mask: Optional[torch.Tensor] = None
+                               ) -> torch.Tensor:
+        """predict_batch as a differentiable layer: returns a fresh [B, 2] actions tensor (not a view of self.actions).
+        When grad is enabled and ref_speed or weights requires grad, the forward pass also runs mpc_sensitivity on the
+        solution (flags into self.sens_flags[:B]) and the backward pass returns J^T grad_out through the parsing of
+        k_prepare (see _param_chain_masks): 0 for a NaN or clipped ref_speed, for weights[:, 0] where a collision forces
+        w_speed, and for every problem whose sensitivity is flagged with more than WEAKLY_ACTIVE."""
+        want = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (ref_speed, weights))
+        return _MpcLayer.apply(self, obs, ref_speed, weights, reset_mask, want)
 
     def prepare_batch(self, obs, ref_speed=None, weights=None, reset_mask=None) -> Dict[str, torch.Tensor]:
         """Parsing + collision logic only (mpc_prepare); returns the parsed-problem workspace as tensors
@@ -641,3 +682,51 @@ class PureMPC_NoCollision_Agent(PureMPC_Agent):
         cfg = dict(cfg)
         cfg.setdefault("weight_speed", cfg.get("weight_state", 1.0) if literal else 1.0)   # quirk Q4
         super().__init__(env, cfg, device, n_starts=n_starts)
+
+
+def _param_chain_masks(ref_speed: Optional[torch.Tensor], is_collide: torch.Tensor, B: int) -> torch.Tensor:
+    """[B, 4] d(vr_b, w_speed, w_control, w_diff) / d(ref_speed, weights[:, 0], weights[:, 1], weights[:, 2]) of
+    k_prepare (csrc/mpc_prepare.cu:438-447): w_speed = 100 when is_collide (:440); vr_b = clip(ref_speed, 0, 30) when
+    ref_speed is not NaN (:446), so the derivative is 1 strictly inside (0, 30) and 0 for NaN or a clipped value."""
+    m = torch.ones(B, 4, dtype=torch.float32, device=is_collide.device)
+    if ref_speed is not None:
+        r = ref_speed.detach().reshape(-1).to(m.device, torch.float32)
+        m[:, 0] = ((r > 0) & (r < 30)).float()
+    m[:, 1] = (is_collide[:B] == 0).float()
+    return m
+
+
+class _MpcLayer(torch.autograd.Function):
+    """BatchedPureMPC.predict_batch_autograd."""
+
+    @staticmethod
+    def forward(ctx, agent, obs, ref_speed, weights, reset_mask, want):
+        B = agent._check_obs(obs)
+        rs = None if ref_speed is None else ref_speed.detach()
+        w = None if weights is None else weights.detach()
+        if not want:                               # grad disabled, or neither input requires it
+            return agent.predict_batch(obs, rs, w, reset_mask).clone()
+        a, U = agent.predict_batch(obs, rs, w, reset_mask, return_controls=True)
+        actions = a.clone()
+        sens = agent.sensitivity(U)
+        agent.sens_flags[:B].copy_(sens["flags"])
+        jac = torch.nan_to_num(sens["jac"], nan=0.0)        # flagged problems: no gradient
+        jac = jac * _param_chain_masks(rs, agent.is_collide, B)[:, None, :]
+        ctx.save_for_backward(jac)
+        ctx.like = (ref_speed, weights)
+        return actions
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        (jac,) = ctx.saved_tensors
+        gp = torch.einsum("brc,br->bc", jac, grad_out.to(jac.dtype))
+        g_rs = g_w = None
+        rs, w = ctx.like
+        if ctx.needs_input_grad[2]:
+            g_rs = gp[:, 0].reshape(rs.shape).to(rs.dtype).to(rs.device)
+        if ctx.needs_input_grad[3]:
+            B = gp.shape[0]
+            g = torch.zeros(B, w.numel() // B, dtype=gp.dtype, device=gp.device)
+            g[:, :3] = gp[:, 1:4]
+            g_w = g.reshape(w.shape).to(w.dtype).to(w.device)
+        return None, None, g_rs, g_w, None, None

@@ -3,7 +3,8 @@
     python mpc-rl_for_avs_b200/build.py [--force] [--verbose]
 
 mpc_prepare.cu is compiled with -fmad=false (its FP64 predicates must round exactly like the numpy
-oracle); everything else with default FMA contraction.
+oracle), mpc_sens.cu too (its FP64 linear algebra stays within rounding of the host build's); everything else
+with default FMA contraction.
 """
 from __future__ import annotations
 
@@ -18,7 +19,8 @@ LIB = os.path.join(HERE, os.environ.get("MPC_LIB_NAME", "libmpcb200.so"))      #
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",
           "--expt-relaxed-constexpr"]
-UNITS = [("mpc_solve.cu", []), ("mpc_prepare.cu", ["-fmad=false"]), ("mpc_capi.cu", []), ("mpc_env.cu", []), ("mpc_kkt.cu", [])]
+UNITS = [("mpc_solve.cu", []), ("mpc_prepare.cu", ["-fmad=false"]), ("mpc_capi.cu", []), ("mpc_env.cu", []), ("mpc_kkt.cu", []),
+         ("mpc_sens.cu", ["-fmad=false"])]
 
 
 def _nvcc() -> str:

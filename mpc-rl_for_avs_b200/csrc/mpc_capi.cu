@@ -562,6 +562,36 @@ MPC_API int mpc_kkt(MpcHandle* h, const MpcProblemBatch* batch, int B, const flo
   return MPC_OK;
 }
 
+MPC_API int mpc_sensitivity(MpcHandle* h, const MpcProblemBatch* batch, int B, const float* U, float act_tol,
+                            float stat_tol, const MpcSensOut* out, void* stream) {
+  if (!h) return MPC_ERR_BAD_ARG;
+  if (!U || !out || !out->jac || !out->flags) return fail(h, MPC_ERR_BAD_ARG, "mpc_sensitivity: U, out->jac and out->flags are required");
+  if (!(act_tol >= 0.f)) return fail(h, MPC_ERR_BAD_ARG, "mpc_sensitivity: act_tol must be >= 0 and not NaN");
+  if (!(stat_tol >= 0.f)) return fail(h, MPC_ERR_BAD_ARG, "mpc_sensitivity: stat_tol must be >= 0 and not NaN");
+  if (B < 0) return fail(h, MPC_ERR_BAD_ARG, "mpc_sensitivity: B < 0");
+  if (B > h->max_batch) return fail(h, MPC_ERR_TOO_LARGE, "mpc_sensitivity: B exceeds max_batch of mpc_create");
+  MpcProblemBatch wb;
+  if (!batch) {
+    if (B != h->last_B) return fail(h, MPC_ERR_BAD_ARG, "mpc_sensitivity: batch == NULL needs the B of the last mpc_prepare / mpc_predict");
+    mpc_workspace_batch(h, &wb);
+    batch = &wb;
+  } else {
+    int rc = check_batch(h, batch, B);
+    if (rc) return rc;
+  }
+  if (B == 0) return MPC_OK;
+  CK(h, cudaSetDevice(h->device));
+  SensLaunch k{};
+  k.batch = *batch; k.B = B; k.N = h->scfg.N; k.M = h->scfg.M;
+  k.dt = prep_dt(h->cfg.dt);
+  k.w_distance = h->scfg.w_distance; k.w_collision = h->scfg.w_collision;
+  k.literal_no_collision = h->scfg.literal_no_collision;
+  k.ref = h->tables.ref; k.U = U; k.act_tol = (double)act_tol; k.stat_tol = (double)stat_tol; k.out = *out;
+  CK(h, launch_sens(k, (cudaStream_t)stream));
+  h->launches += 1;
+  return MPC_OK;
+}
+
 MPC_API int mpc_set_warm_start(MpcHandle* h, const float* u_init) {
   if (!h) return MPC_ERR_BAD_ARG;
   h->u_init = u_init;

@@ -123,4 +123,18 @@ struct KktLaunch {
 };
 cudaError_t launch_kkt(const KktLaunch& k, cudaStream_t stream);
 
+// defined in mpc_sens.cu: the sensitivity dU_0/dp of controls U (mpc_sensitivity)
+struct SensLaunch {
+  MpcProblemBatch batch;
+  int B, N, M;
+  double dt;              // the double 1 / policy_frequency
+  double w_distance, w_collision;
+  int literal_no_collision;
+  const double* ref;      // RefTables::ref
+  const float* U;         // [B][N][2]
+  double act_tol, stat_tol;
+  MpcSensOut out;
+};
+cudaError_t launch_sens(const SensLaunch& s, cudaStream_t stream);
+
 }  // namespace mpcb
